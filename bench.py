@@ -2,7 +2,7 @@
 """bench.py — phased windows/s of the per-window phasing hot path on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload exome|chr22|hypermutated|normal|filter]
+                    [--workload exome|chr22|hypermutated|normal|filter] [--dump-outputs DIR]
 
 Default workload (config.workload): one whole-exome-shaped shard per GPU — BASELINE.json configs[2]
 ("synthetic whole exome (~20k transcripts), 100x tumor BAM, somatic mode"): 20 000 single-transcript
@@ -27,6 +27,11 @@ A step = one pass of the hot path over the shard.
   cpu_baseline : the CPU oracle (a restatement of the reference's Rust code, which cannot be built
           here — no cargo/rustc) on one core over a bounded sample of the same workload.
 `--impl reference` times that oracle on all host cores instead.
+
+`--dump-outputs DIR` writes what the last timed step computed (rank 0) as DIR/<name>.npy: the records of
+mph_phase_resident (a fixed, seeded sample when there are more than DUMP_RECORDS; every field, strings as byte
+values with a length per record) or the hit flags of the filter probe. The inputs are seeded, so two builds
+can be compared array for array.
 """
 import argparse
 import json
@@ -197,6 +202,41 @@ def aggregate_over_ranks(dist, device, dev_ms, e2e_ms, windows, read_windows):
 
 KERNEL_KEYS = ("k1_ms", "replay_ms", "k2_ms", "k3_ms", "k4_ms", "k5_ms")
 
+DUMP_RECORDS = 16384  # records sampled for --dump-outputs; keeps the dump of every workload well under DUMP_LIMIT
+DUMP_LIMIT = 64 << 20
+
+
+def write_dump(out_dir, arrays):
+    import numpy as np
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit("--dump-outputs: %d bytes exceed the %d byte limit" % (total, DUMP_LIMIT))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def dump_records(res, out_dir):
+    """Every field of the records a caller of the path receives (mph_record): numbers as float64, each string field as
+    its bytes (float32, concatenated) plus <field>_len (float64, -1 for NULL). More than DUMP_RECORDS records are sampled
+    with a fixed seed; record_index holds the sampled positions and n_records the full count."""
+    import ctypes
+    import numpy as np
+    import microphaser_b200 as m
+    n = len(res)
+    idx = np.arange(n) if n <= DUMP_RECORDS else np.sort(np.random.default_rng(SEED).choice(n, DUMP_RECORDS, replace=False))
+    recs = [res.record(int(i)) for i in idx]
+    arrays = {"n_records": np.array([n], dtype=np.float64), "record_index": idx.astype(np.float64)}
+    for f, typ in m.Record._fields_:
+        vals = [r[f] for r in recs]
+        if typ is ctypes.c_char_p:
+            raw = [None if v is None else v.encode() for v in vals]
+            arrays[f + "_len"] = np.array([-1 if b is None else len(b) for b in raw], dtype=np.float64)
+            arrays[f] = np.frombuffer(b"".join(b or b"" for b in raw), dtype=np.uint8).astype(np.float32)
+        else:
+            arrays[f] = np.array(vals, dtype=np.float64)
+    write_dump(out_dir, arrays)
+
 
 def filter_workload(args, rank, local_rank, world, dist, barrier):
     """BASELINE.json configs[4]b: ref_set.contains(peptide) for 1 M neopeptides (reference src/peptides.rs:502,684)."""
@@ -221,6 +261,8 @@ def filter_workload(args, rank, local_rank, world, dist, barrier):
         if i >= args.warmup:
             ms.append(dt)
             kern.append(ctx.timing()["k1_ms"])
+    if args.dump_outputs and rank == 0:
+        write_dump(args.dump_outputs, {"hits": hits.astype(np.float32)})
     ref_set = set(map(bytes, ref[:200000]))
     sample = queries[:5000]
     for q, h in zip(sample, hits[:5000]):
@@ -255,7 +297,12 @@ def main():
     ap.add_argument("--cpu-sample-transcripts", type=int, default=1000)
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the oracle run (and with it the parity check and e2e_files)")
     ap.add_argument("--e2e-steps", type=int, default=0, help="end-to-end calls to time (default: --steps)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the CUDA path; the reference arm writes files only")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -339,6 +386,8 @@ def main():
     res = ctx.collect()
     t_res = ctx.timing()
     n_records = len(res)
+    if args.dump_outputs and rank == 0:
+        dump_records(res, args.dump_outputs)
     res.close()
     windows, read_windows = t_res["windows"], t_res["read_windows"]
     dev_ms = chain_ms / args.steps
