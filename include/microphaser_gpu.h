@@ -183,7 +183,10 @@ int mph_result_write(const mph_result* r, int fd_fasta, int fd_tsv, int fd_norma
 
 /* ---- file-level driver: replaces microphasing::phase (src/microphasing.rs:1943-2131) ------ */
 /* `somatic` sub-command on real files; GTF is read from gtf_path ("-" = stdin), mutant FASTA goes
- * to fasta_out_path ("-" = stdout). */
+ * to fasta_out_path ("-" = stdout). With a BAM index next to the BAM (<bam>.bai, else <bam minus .bam>.bai)
+ * the reads are fetched through it gene range by gene range and phased in shards as they close, so host
+ * memory follows the shard size; a malformed index is MPH_ERR_INPUT. Without one the whole BAM is loaded
+ * first. */
 int mph_run_somatic(mph_ctx* ctx, const char* bam_path, const char* ref_path, const char* variants_path, const char* gtf_path,
                     const char* fasta_out_path, const char* tsv_path, const char* normal_path, uint32_t window_len,
                     int unsupported_allele_warning_only);
@@ -194,7 +197,8 @@ int mph_run_normal(mph_ctx* ctx, const char* bam_path, const char* ref_path, con
 
 /* the same over several devices of one box: genes are split into n_ctx contiguous ranges balanced by
  * read count, every context phases its range on its own host thread, records are concatenated in
- * range order. No collective is involved (shards are independent). */
+ * range order. With a BAM index the streamed shards go to whichever device is free as they close.
+ * No collective is involved (shards are independent). */
 int mph_run_somatic_multi(mph_ctx* const* ctxs, int n_ctx, const char* bam_path, const char* ref_path, const char* variants_path,
                           const char* gtf_path, const char* fasta_out_path, const char* tsv_path, const char* normal_path,
                           uint32_t window_len, int unsupported_allele_warning_only);

@@ -1491,6 +1491,151 @@ int mph_result_write(const mph_result* r, int fd_fasta, int fd_tsv, int fd_norma
   });
 }
 
+static void add_timing(mph_timing& a, const mph_timing& t) {
+  a.h2d_ms += t.h2d_ms; a.k1_ms += t.k1_ms; a.k2_ms += t.k2_ms; a.k3_ms += t.k3_ms; a.k4_ms += t.k4_ms; a.d2h_ms += t.d2h_ms;
+  a.residue_ms += t.residue_ms; a.total_ms += t.total_ms; a.replay_ms += t.replay_ms; a.k5_ms += t.k5_ms; a.pack_ms += t.pack_ms; a.kernels_ms += t.kernels_ms; a.h2d_bytes += t.h2d_bytes; a.d2h_bytes += t.d2h_bytes;
+  a.windows += t.windows; a.read_windows += t.read_windows; a.windows_enumerated += t.windows_enumerated; a.n_interesting += t.n_interesting;
+  a.n_records += t.n_records; a.kernel_launches += t.kernel_launches; a.n_replay_units += t.n_replay_units;
+}
+
+// Genes of an indexed BAM: this thread walks the GTF and fetches gene by gene in the reference's one-pass order
+// (reference slice, reads, variants), closing a shard every `reads_per_shard` reads (MPH_SHARD_READS overrides it). A pool
+// of workers packs each closed shard and phases it on whichever device is free; shards are written in order as they
+// complete. The walk waits while workers + 1 shards are fetched but not yet written, so the reads held in memory follow
+// the shard size, not the file size. A failure of the walk (a corrupt block late in the BAM) is reported after the
+// shards before it are written, as the reference, which streams, does.
+static void run_streamed(const std::vector<mph_ctx*>& ctxs, std::istream& gtf, mphio::BamFile& bam, const mphio::BamIndex& index,
+                         mphio::VcfFile& vcf, mphio::FastaIndexed& fasta, const IngestOptions& io, int fd_fa, int fd_tsv, int fd_n) {
+  const auto t_fetch0 = std::chrono::steady_clock::now();
+  std::vector<ParsedGene> parsed = read_gtf(gtf, io.mode);  // the unsorted-GTF panic comes before any output
+  const size_t n_dev = ctxs.size();
+  size_t per_dev = std::min<size_t>(12, std::max<size_t>(1, std::thread::hardware_concurrency() / n_dev));
+  if (const char* e = getenv("MPH_PACK_THREADS")) per_dev = size_t(std::max(1, atoi(e)));
+  uint64_t reads_per_shard = io.mode == 1 ? 2000000ull : 8000000ull;
+  if (const char* e = getenv("MPH_SHARD_READS")) reads_per_shard = uint64_t(std::max(1, atoi(e)));
+  const size_t n_workers = n_dev * per_dev;
+  std::mutex mu;
+  std::condition_variable cv;
+  std::deque<std::pair<size_t, std::vector<GeneInput>>> queue;  // closed shards waiting for a worker
+  std::map<size_t, mph_result*> results;                          // phased shards waiting for their turn to be written
+  size_t n_closed = 0, next_out = 0;
+  bool fetch_done = false;
+  int hw = 0;
+  std::exception_ptr first_err;
+  std::vector<std::mutex> dev_mu(n_dev);
+  std::vector<mph_timing> acc(n_dev, mph_timing{});
+  std::atomic<uint64_t> pack_us{0}, write_us{0};
+  auto worker = [&](size_t w) {
+    for (;;) {
+      std::pair<size_t, std::vector<GeneInput>> job;
+      {
+        std::unique_lock<std::mutex> lk(mu);
+        cv.wait(lk, [&] { return !queue.empty() || fetch_done; });
+        if (queue.empty()) return;
+        job = std::move(queue.front());
+        queue.pop_front();
+      }
+      const size_t k = job.first;
+      mph_result* res = nullptr;
+      std::exception_ptr err;
+      try {
+        bool skip;
+        {
+          std::lock_guard<std::mutex> lk(mu);
+          skip = first_err != nullptr;
+        }
+        if (!skip) {
+          const auto tp0 = std::chrono::steady_clock::now();
+          Packer packer(io.window_len, io.mode);
+          pack_genes(job.second, 0, job.second.size(), packer);
+          std::vector<GeneInput>().swap(job.second);  // the reads' batches are free once packed
+          std::unique_ptr<mph_batch> batch(new mph_batch);
+          batch->b = std::move(packer.batch());
+          finish_batch(batch.get(), false);
+          pack_us += uint64_t(std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now() - tp0).count());
+          // a context is not re-entrant: the first free device, else this worker's own
+          size_t dv = n_dev;
+          for (size_t d = 0; d < n_dev && dv == n_dev; ++d)
+            if (dev_mu[d].try_lock()) dv = d;
+          if (dv == n_dev) {
+            dv = w % n_dev;
+            dev_mu[dv].lock();
+          }
+          std::lock_guard<std::mutex> dl(dev_mu[dv], std::adopt_lock);
+          phase_batch_impl(ctxs[dv], batch.get(), &res);
+          add_timing(acc[dv], ctxs[dv]->timing);
+        }
+      } catch (...) {
+        err = std::current_exception();
+      }
+      // ordered concatenation: shard k goes out when shards 0 .. k-1 are out; after a failure nothing later is written
+      std::lock_guard<std::mutex> lk(mu);
+      if (err && !first_err) first_err = err;
+      results[k] = res;
+      for (auto it = results.find(next_out); it != results.end(); it = results.find(next_out)) {
+        if (it->second) {
+          const auto tw0 = std::chrono::steady_clock::now();
+          if (!first_err && mph_result_write(it->second, fd_fa, fd_tsv, fd_n, &hw) != MPH_OK && !first_err)
+            first_err = std::make_exception_ptr(std::runtime_error(g_last_error));
+          write_us += uint64_t(std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now() - tw0).count());
+          delete it->second;
+        }
+        results.erase(it);
+        ++next_out;
+      }
+      cv.notify_all();
+    }
+  };
+  std::vector<std::thread> pool;
+  for (size_t w = 0; w < n_workers; ++w) pool.emplace_back(worker, w);
+  std::exception_ptr fetch_err;
+  try {
+    ReadBuffer reads(bam, index);
+    VariantBuffer variants(vcf);
+    std::vector<GeneInput> shard;
+    uint64_t shard_reads = 0;
+    auto close_shard = [&] {
+      std::unique_lock<std::mutex> lk(mu);
+      cv.wait(lk, [&] { return n_closed - next_out < n_workers + 1 || first_err; });
+      queue.emplace_back(n_closed++, std::move(shard));
+      shard.clear();
+      shard_reads = 0;
+      cv.notify_all();
+    };
+    try {
+      for (ParsedGene& pg : parsed) {
+        if (pg.biotype != "protein_coding") continue;  // :1964
+        {
+          std::lock_guard<std::mutex> lk(mu);
+          if (first_err) break;
+        }
+        shard.push_back(fetch_gene(std::move(pg.gene), reads, variants, vcf, fasta, io));
+        shard_reads += shard.back().n_reads;
+        if (shard_reads >= reads_per_shard) close_shard();
+      }
+    } catch (...) {
+      fetch_err = std::current_exception();  // the genes fetched before the failure are still phased and written
+    }
+    if (!shard.empty()) close_shard();
+  } catch (...) {
+    if (!fetch_err) fetch_err = std::current_exception();
+  }
+  const double fetch_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_fetch0).count();
+  {
+    std::lock_guard<std::mutex> lk(mu);
+    fetch_done = true;
+  }
+  cv.notify_all();
+  for (auto& t : pool) t.join();
+  for (auto& kv : results) delete kv.second;
+  for (size_t dv = 0; dv < n_dev; ++dv) ctxs[dv]->timing = acc[dv];
+  ctxs[0]->timing.ingest_ms = fetch_ms;
+  ctxs[0]->timing.pack_ms = double(pack_us.load()) / 1000.0;
+  ctxs[0]->timing.write_ms = double(write_us.load()) / 1000.0;
+  if (first_err) std::rethrow_exception(first_err);
+  if (fetch_err) std::rethrow_exception(fetch_err);
+}
+
 // shared by the single- and multi-device file drivers
 static void run_somatic_files(const std::vector<mph_ctx*>& ctxs, const char* bam_path, const char* ref_path, const char* variants_path,
                               const char* gtf_path, const char* fasta_out_path, const char* tsv_path, const char* normal_path,
@@ -1522,7 +1667,12 @@ static void run_somatic_files(const std::vector<mph_ctx*>& ctxs, const char* bam
       if (const char* bb = getenv("MPH_GPU_INFLATE_BLOCKS")) inflater.batch_blocks = size_t(std::max(256, atoi(bb)));
     }
   }
-  mphio::BamFile bam(bam_path, io_threads, inflater);
+  // with an index next to the BAM the genes are streamed: reads are fetched through the index, and batches of 64 blocks
+  // keep the read-ahead that a seek throws away small
+  const std::string bai = mphio::BamIndex::locate(bam_path);
+  mphio::BamFile bam(bam_path, io_threads, inflater, bai.empty() ? 256 : 64);
+  std::unique_ptr<mphio::BamIndex> index;
+  if (!bai.empty()) index.reset(new mphio::BamIndex(bai, bam.ref_names.size(), bam.file_bytes()));
   mphio::VcfFile vcf(variants_path);
   mphio::FastaIndexed fasta(ref_path);
   // the reference creates its output files before it starts phasing (src/main.rs:79-85)
@@ -1552,6 +1702,14 @@ static void run_somatic_files(const std::vector<mph_ctx*>& ctxs, const char* bam
       gf.open(gtf_path);
       if (!gf) throw std::runtime_error(std::string("cannot open ") + gtf_path);
       gin = &gf;
+    }
+    if (index) {
+      run_streamed(ctxs, *gin, bam, *index, vcf, fasta, io, fd_fa, fd_tsv, fd_n);
+      if (gpu_inflate && getenv("MPH_IO_TRACE"))
+        fprintf(stderr, "[mph io] device inflate: %zu batches, %.1f MB in, %.1f MB out, %.1f ms inside the inflater (copies + kernel)%s\n", gpu_inflate->batches,
+                gpu_inflate->bytes_in / 1e6, gpu_inflate->bytes_out / 1e6, gpu_inflate->ms_total, bam.device_inflate_used() ? "" : " - not used (small file or fallback to zlib)");
+      close_all();
+      return;
     }
     const auto t_ingest0 = std::chrono::steady_clock::now();
     ReadBufferLoader loader(bam);  // the BAM loads on its own thread while this one parses the GTF and fetches reference slices and variants
@@ -1585,12 +1743,6 @@ static void run_somatic_files(const std::vector<mph_ctx*>& ctxs, const char* bam
     int hw = 0;
     std::exception_ptr first_err;
     std::vector<mph_timing> acc(n_dev, mph_timing{});  // a device's timing is the sum over its shards
-    auto add_timing = [](mph_timing& a, const mph_timing& t) {
-      a.h2d_ms += t.h2d_ms; a.k1_ms += t.k1_ms; a.k2_ms += t.k2_ms; a.k3_ms += t.k3_ms; a.k4_ms += t.k4_ms; a.d2h_ms += t.d2h_ms;
-      a.residue_ms += t.residue_ms; a.total_ms += t.total_ms; a.replay_ms += t.replay_ms; a.k5_ms += t.k5_ms; a.pack_ms += t.pack_ms; a.kernels_ms += t.kernels_ms; a.h2d_bytes += t.h2d_bytes; a.d2h_bytes += t.d2h_bytes;
-      a.windows += t.windows; a.read_windows += t.read_windows; a.windows_enumerated += t.windows_enumerated; a.n_interesting += t.n_interesting;
-      a.n_records += t.n_records; a.kernel_launches += t.kernel_launches; a.n_replay_units += t.n_replay_units;
-    };
     // ordered concatenation: shard k goes out when shards 0 .. k-1 are out; the TSV header goes out with the first row only.
     // After a failure nothing later than the failing shard is written (the reference stops at that point, too).
     auto shard_finished = [&](size_t k, std::exception_ptr err) {

@@ -16,6 +16,7 @@
 #include <istream>
 #include <memory>
 
+#include "../io/bam_index.hpp"
 #include "../io/hts_io.hpp"
 #include "batch.hpp"
 
@@ -27,7 +28,7 @@ inline uint64_t fnv1a(const std::string& s) {
   return h;
 }
 
-// bam::RecordBuffer::fetch over a coordinate-sorted BAM held in memory per contig
+// bam::RecordBuffer::fetch over a coordinate-sorted BAM: held in memory per contig, or read through its index
 class ReadBuffer {
  public:
   // one alignment record. Sequence and qualities are NOT copied: the pointers go into the inflated BGZF batches, which the
@@ -77,6 +78,16 @@ class ReadBuffer {
     }
     index_by_tid();
   }
+
+  // Indexed mode: nothing is loaded up front. A re-fetch finds where to start through the index - a seek, or a read
+  // forward when that start lies a little ahead of what has been read - and every fetch reads on lazily, only as far as
+  // its end plus the one overflow record. Records point into the inflated batches; a batch is dropped by the buffer once
+  // no record of the current fetch lies in it, and freed once no gene pins it (pins()).
+  ReadBuffer(mphio::BamFile& bam, const mphio::BamIndex& index)
+      : bam_(bam), index_(&index), read_on_bytes_(bam.inflate_threads() > 1 ? uint64_t(4) << 20 : uint64_t(64) << 10) {}
+
+  // keeps an inflated batch alive
+  using Pin = std::shared_ptr<const void>;
 
  private:
   // a growable array whose new elements are NOT value-initialised: the loader overwrites every byte it adds, and
@@ -501,9 +512,10 @@ class ReadBuffer {
       size_t size() const { return n; }
       const Rec& operator[](size_t i) const { return p[i]; }
     };
-    const View v{recs_.data() + tid_range_[size_t(tid)].first, tid_range_[size_t(tid)].second - tid_range_[size_t(tid)].first};
     const bool refetch = inner_.empty() || uint64_t(inner_.back()->pos) < start || inner_.front()->tid != tid ||
                          uint64_t(inner_.front()->pos) > start;
+    if (index_) return fetch_indexed(tid, start, end, refetch);
+    const View v{recs_.data() + tid_range_[size_t(tid)].first, tid_range_[size_t(tid)].second - tid_range_[size_t(tid)].first};
     if (refetch) {
       inner_.clear();
       tid_ = tid;
@@ -523,7 +535,170 @@ class ReadBuffer {
     return inner_;
   }
 
+  // indexed mode: the batches the records of the last fetch (and its overflow record) point into; empty otherwise
+  std::vector<Pin> pins() const { return std::vector<Pin>(live_.begin(), live_.begin() + long(std::min(live_.size(), bi_ + 1))); }
+
  private:
+  // ---- indexed mode
+  // one inflated batch and the records that start in it; a record that began in the previous batch is completed in `head`
+  struct Block {
+    mphio::RawBytes data;
+    std::vector<uint8_t> head;
+    std::vector<Rec> recs;
+    std::vector<uint64_t> voff;  // virtual offset of each record
+    std::unique_ptr<uint32_t[]> cig;
+  };
+
+  const std::deque<const Rec*>& fetch_indexed(int tid, uint64_t start, uint64_t end, bool refetch) {
+    if (refetch) {
+      inner_.clear();
+      tid_ = tid;
+      position(index_->first_offset(tid, int64_t(std::min<uint64_t>(start, uint64_t(INT64_MAX)))));
+    } else {
+      while (!inner_.empty() && uint64_t(inner_.front()->pos) < start) inner_.pop_front();
+    }
+    // the whole-file loop over the contig's records, which end where the next contig's begin
+    for (const Rec* r; (r = peek()) && r->tid == tid_;) {
+      ++ri_;
+      if (r->is_unmapped()) continue;
+      const uint64_t pos = uint64_t(r->pos);
+      if (pos >= end) { overflow_ = r; break; }
+      if (pos >= start || (refetch && uint64_t(r->end) > start)) inner_.push_back(r);
+    }
+    // batches before the one holding the earliest record still needed go (the genes that point into them pin them)
+    const Rec* keep = !inner_.empty() ? inner_.front() : overflow_;
+    size_t b = bi_;
+    for (size_t i = 0; keep && i < bi_; ++i)
+      if (keep >= live_[i]->recs.data() && keep < live_[i]->recs.data() + live_[i]->recs.size()) { b = i; break; }
+    live_.erase(live_.begin(), live_.begin() + long(std::min(b, live_.size())));
+    bi_ -= std::min(b, bi_);
+    return inner_;
+  }
+
+  // moves the cursor to the first record at or after virtual offset t (BamIndex::NONE: the contig has none to give)
+  void position(uint64_t t) {
+    contig_done_ = t == mphio::BamIndex::NONE;
+    if (contig_done_) return;
+    if (!live_.empty() && !live_.front()->voff.empty() && t >= live_.front()->voff.front() && t < stream_voff_) {
+      for (size_t b = 0; b < live_.size(); ++b) {  // among the records read since the last seek
+        const auto& v = live_[b]->voff;
+        auto it = std::lower_bound(v.begin(), v.end(), t);
+        if (it != v.end()) { bi_ = b; ri_ = size_t(it - v.begin()); return; }
+      }
+    }
+    live_.clear();
+    bi_ = ri_ = 0;
+    if (!eof_ && t >= stream_voff_ && (t >> 16) - (stream_voff_ >> 16) <= read_on_bytes_) {
+      while (read_block()) {
+        const auto& v = live_.back()->voff;
+        auto it = std::lower_bound(v.begin(), v.end(), t);
+        if (it != v.end()) {
+          live_.erase(live_.begin(), live_.end() - 1);
+          ri_ = size_t(it - v.begin());
+          return;
+        }
+      }
+      live_.clear();  // no record at or after t
+      return;
+    }
+    carry_.clear();
+    eof_ = false;
+    try {
+      bam_.seek(t);
+    } catch (const mphio::IoError& e) {
+      throw mphio::IoError(std::string(e.what()) + " (offset from " + index_->path() + ")");
+    }
+    stream_voff_ = t;
+  }
+
+  // the record under the cursor, reading on as needed; nullptr at the end of the file or of a contig without records
+  const Rec* peek() {
+    if (contig_done_) return nullptr;
+    for (;;) {
+      if (bi_ < live_.size()) {
+        if (ri_ < live_[bi_]->recs.size()) return &live_[bi_]->recs[ri_];
+        if (bi_ + 1 < live_.size()) { ++bi_; ri_ = 0; continue; }
+      }
+      if (!read_block()) return nullptr;
+    }
+  }
+
+  // frames and decodes the next inflated batch into a block at the end of live_; false at the end of the file
+  bool read_block() {
+    if (eof_) return false;
+    std::shared_ptr<Block> blk(new Block);
+    size_t o = 0;
+    std::vector<mphio::BgzfSpan> spans;
+    if (!bam_.next_chunk(blk->data, o, spans)) {
+      eof_ = true;
+      if (!carry_.empty()) throw mphio::IoError("truncated BAM record");
+      return false;
+    }
+    const uint8_t* base = blk->data.data();
+    const size_t size = blk->data.size();
+    size_t si = 0;
+    auto voff_at = [&](size_t at) {
+      while (si + 1 < spans.size() && spans[si + 1].ooff <= int64_t(at)) ++si;
+      return spans[si].coff << 16 | uint64_t(int64_t(at) - spans[si].ooff);
+    };
+    std::vector<std::pair<const uint8_t*, uint64_t>> at;  // record bytes after the length prefix, virtual offset
+    size_t n_cig = 0;
+    auto frame = [&](const uint8_t* p, size_t avail, uint64_t voff) -> size_t {  // 0: incomplete
+      if (avail < 4) return 0;
+      int32_t bs;
+      memcpy(&bs, p, 4);
+      if (bs < 32) throw mphio::IoError("corrupt BAM record");
+      if (avail < 4 + size_t(bs)) return 0;
+      uint16_t nc;
+      memcpy(&nc, p + 16, 2);
+      if (32 + 4 * size_t(nc) > size_t(bs)) throw mphio::IoError("corrupt BAM record");
+      n_cig += nc;
+      at.emplace_back(p + 4, voff);
+      return 4 + size_t(bs);
+    };
+    if (!carry_.empty()) {  // the record that began in the previous batch: its length prefix first, then the rest
+      size_t take = std::min(size_t(4) - std::min<size_t>(4, carry_.size()), size - o);
+      carry_.insert(carry_.end(), base + o, base + o + take);
+      o += take;
+      if (carry_.size() >= 4) {
+        int32_t bs;
+        memcpy(&bs, carry_.data(), 4);
+        if (bs < 32) throw mphio::IoError("corrupt BAM record");
+        take = std::min(4 + size_t(bs) - carry_.size(), size - o);
+        carry_.insert(carry_.end(), base + o, base + o + take);
+        o += take;
+        if (carry_.size() == 4 + size_t(bs)) {
+          blk->head.swap(carry_);
+          carry_.clear();
+          frame(blk->head.data(), blk->head.size(), carry_voff_);
+        }
+      }
+    }
+    while (carry_.empty()) {
+      const size_t n = frame(base + o, size - o, voff_at(o));
+      if (!n) break;
+      o += n;
+    }
+    if (carry_.empty() && o < size) {
+      carry_voff_ = voff_at(o);
+      carry_.assign(base + o, base + size);
+    }
+    stream_voff_ = carry_.empty() ? voff_at(size) : carry_voff_;
+    blk->recs.resize(at.size());
+    blk->voff.resize(at.size());
+    blk->cig.reset(new uint32_t[n_cig + 1]);
+    uint32_t* cig = blk->cig.get();
+    for (size_t i = 0; i < at.size(); ++i) {
+      int32_t bs;
+      memcpy(&bs, at[i].first - 4, 4);
+      decode_record(at[i].first, bs, cig, blk->recs[i]);
+      cig += blk->recs[i].n_cigar;
+      blk->voff[i] = at[i].second;
+    }
+    live_.push_back(std::move(blk));
+    return true;
+  }
+
   static uint64_t fnv1a_bytes(const char* p, size_t n) {
     uint64_t h = 1469598103934665603ull;
     for (size_t i = 0; i < n; ++i) { h ^= uint8_t(p[i]); h *= 1099511628211ull; }
@@ -541,6 +716,16 @@ class ReadBuffer {
   const Rec* overflow_ = nullptr;
   int tid_ = -1;
   size_t cur_ = 0;
+  // indexed mode
+  const mphio::BamIndex* index_ = nullptr;
+  // A start at most this many compressed bytes ahead of what has been read is reached by reading on instead of a seek.
+  // A seek of the sequential reader costs nothing, one of the threaded reader throws away its read-ahead (three batches).
+  uint64_t read_on_bytes_ = 0;
+  std::deque<std::shared_ptr<Block>> live_;  // the batches read since the last seek that may still be needed
+  size_t bi_ = 0, ri_ = 0;                    // cursor: block in live_, record in it
+  std::vector<uint8_t> carry_;                // the head of a record whose tail is in the next batch
+  uint64_t carry_voff_ = 0, stream_voff_ = 0; // its virtual offset; that of the first byte not yet framed
+  bool eof_ = false, contig_done_ = false;
 };
 
 // bcf::Reader (streaming) + bcf::buffer::RecordBuffer::fetch
@@ -756,6 +941,7 @@ struct GeneInput {
   // lazy form (file drivers): the buffered records themselves; `reads` is built from them when the gene is packed, which
   // happens on the packing threads instead of the single thread that walks the GTF
   std::vector<const ReadBuffer::Rec*> recs;
+  std::vector<ReadBuffer::Pin> pins;  // indexed mode: the inflated batches `recs` point into, released once packed
   size_t n_reads = 0;
   uint32_t max_read_len = 0;
   void materialize() {
@@ -778,6 +964,41 @@ struct GeneInput {
   std::vector<std::vector<HostVariant>> sites;
   std::vector<uint8_t> refseq;
 };
+
+// the buffered reads of the gene that pass the mapq filter (:905-920)
+inline void fetch_reads(GeneInput& gi, ReadBuffer& reads, const IngestOptions& opt) {
+  const HostGene& g = gi.gene;
+  const auto& rb = reads.fetch(g.chrom, g.start, g.end);
+  gi.recs.reserve(rb.size());
+  for (auto& rec : rb) {
+    if (rec->mapq < opt.min_mapq) continue;
+    if (rec->l_seq > gi.max_read_len) gi.max_read_len = rec->l_seq;
+    gi.recs.push_back(rec);
+  }
+  gi.n_reads = gi.recs.size();
+  gi.pins = reads.pins();
+}
+
+// variant_tree.insert(rec.pos(), Variant::new(rec)): a later record at the same position replaces the earlier (:937)
+inline void fetch_variants(GeneInput& gi, VariantBuffer& variants, const mphio::VcfFile& vcf, const IngestOptions& opt) {
+  const HostGene& g = gi.gene;
+  std::map<uint32_t, std::vector<HostVariant>> tree;
+  for (auto& rec : variants.fetch(g.chrom, g.start, g.end)) tree[uint32_t(rec.pos)] = alleles_of(vcf, rec, opt.warn_only);
+  for (auto& kv : tree)
+    if (!kv.second.empty()) gi.sites.push_back(std::move(kv.second));
+}
+
+// One gene in the reference's one-pass order (:894-942): reference slice, reads, variants. The indexed paths fetch gene
+// by gene like this, so that nothing of a gene is held longer than it takes to pack it.
+inline GeneInput fetch_gene(HostGene&& g, ReadBuffer& reads, VariantBuffer& variants, const mphio::VcfFile& vcf, mphio::FastaIndexed& fasta,
+                            const IngestOptions& opt) {
+  GeneInput gi;
+  gi.gene = std::move(g);
+  fasta.fetch(gi.gene.chrom, gi.gene.start, uint64_t(gi.gene.end) + 100, gi.refseq);  // end_overflow (:895-901)
+  fetch_reads(gi, reads, opt);
+  fetch_variants(gi, variants, vcf, opt);
+  return gi;
+}
 
 // Streams the GTF and fetches reads / variants / reference for every protein-coding gene, in GTF order.
 // `reads_ready()` returns the loaded ReadBuffer, blocking until it is there: the file drivers load the BAM on another thread
@@ -808,11 +1029,7 @@ inline std::vector<GeneInput> ingest_genes_with(std::istream& gtf, ReadsReady&& 
     try {
       fasta.fetch(g.chrom, g.start, uint64_t(g.end) + 100, gi.refseq);  // end_overflow (:895-901)
       stage = 2;
-      // variant_tree.insert(rec.pos(), Variant::new(rec)): a later record at the same position replaces the earlier (:937)
-      std::map<uint32_t, std::vector<HostVariant>> tree;
-      for (auto& rec : variants.fetch(g.chrom, g.start, g.end)) tree[uint32_t(rec.pos)] = alleles_of(vcf, rec, opt.warn_only);
-      for (auto& kv : tree)
-        if (!kv.second.empty()) gi.sites.push_back(std::move(kv.second));
+      fetch_variants(gi, variants, vcf, opt);
     } catch (...) {
       stashed = std::current_exception();
       stash_gene = out.size();
@@ -825,16 +1042,8 @@ inline std::vector<GeneInput> ingest_genes_with(std::istream& gtf, ReadsReady&& 
   ReadBuffer& reads = reads_ready();
   for (size_t i = 0; i < out.size(); ++i) {
     GeneInput& gi = out[i];
-    const HostGene& g = gi.gene;
     if (i == stash_gene && stash_stage == 0) std::rethrow_exception(stashed);
-    const auto& rb = reads.fetch(g.chrom, g.start, g.end);
-    gi.recs.reserve(rb.size());
-    for (auto& rec : rb) {
-      if (rec->mapq < opt.min_mapq) continue;
-      if (rec->l_seq > gi.max_read_len) gi.max_read_len = rec->l_seq;
-      gi.recs.push_back(rec);
-    }
-    gi.n_reads = gi.recs.size();
+    fetch_reads(gi, reads, opt);
     if (!lazy_reads) gi.materialize();
     if (i == stash_gene) std::rethrow_exception(stashed);
   }
@@ -895,12 +1104,27 @@ inline void pack_genes(std::vector<GeneInput>& genes, size_t lo, size_t hi, Pack
     gi.materialize();
     packer.add_gene(gi.gene, gi.reads, gi.max_read_len, gi.sites, std::move(gi.refseq));
     std::vector<HostRead>().swap(gi.reads);
+    std::vector<ReadBuffer::Pin>().swap(gi.pins);  // the packer copied what it ships
   }
 }
 
-// Builds the batch for every protein-coding gene of the GTF, in GTF order.
+// Builds the batch for every protein-coding gene of the GTF, in GTF order. With an index next to the BAM the reads are
+// fetched through it gene by gene; without one the whole file is loaded first.
 inline void ingest(std::istream& gtf, mphio::BamFile& bam, mphio::VcfFile& vcf, mphio::FastaIndexed& fasta, const IngestOptions& opt,
                    Packer& packer) {
+  const std::string bai = mphio::BamIndex::locate(bam.path());
+  if (!bai.empty()) {
+    const mphio::BamIndex index(bai, bam.ref_names.size(), bam.file_bytes());
+    ReadBuffer reads(bam, index);
+    VariantBuffer variants(vcf);
+    std::vector<GeneInput> one(1);
+    for (ParsedGene& pg : read_gtf(gtf, opt.mode)) {
+      if (pg.biotype != "protein_coding") continue;  // :1964
+      one[0] = fetch_gene(std::move(pg.gene), reads, variants, vcf, fasta, opt);
+      pack_genes(one, 0, 1, packer);
+    }
+    return;
+  }
   ReadBufferLoader loader(bam);
   std::vector<GeneInput> genes = ingest_genes_with(gtf, [&]() -> ReadBuffer& { return loader.get(); }, vcf, fasta, opt, true);
   pack_genes(genes, 0, genes.size(), packer);

@@ -91,6 +91,12 @@ struct BgzfInflaterSpec {
   BgzfBatchInflater fn;
   size_t batch_blocks = 4096, min_bytes = size_t(8) << 20;
 };
+// where the blocks of a handed-over chunk came from: the block at file offset `coff` starts at chunk offset `ooff`, so a
+// byte at chunk offset o has the virtual offset coff << 16 | (o - ooff) of the last span with ooff <= o
+struct BgzfSpan {
+  uint64_t coff;
+  int64_t ooff;
+};
 
 class BgzfReader {
  public:
@@ -98,8 +104,9 @@ class BgzfReader {
   using BatchInflater = BgzfBatchInflater;
   using InflaterSpec = BgzfInflaterSpec;
 
-  explicit BgzfReader(const std::string& path, unsigned threads = 1, InflaterSpec inflater = InflaterSpec())
-      : path_(path), threads_(threads ? threads : 1) {
+  // batch_blocks: BGZF blocks per batch of the threaded reader (read-ahead is up to three batches)
+  explicit BgzfReader(const std::string& path, unsigned threads = 1, InflaterSpec inflater = InflaterSpec(), size_t batch_blocks = 256)
+      : path_(path), threads_(threads ? threads : 1), batch_blocks_(std::max<size_t>(1, batch_blocks)) {
     f_ = fopen(path.c_str(), "rb");
     if (!f_) throw IoError("cannot open " + path);
     if (fseek(f_, 0, SEEK_END) == 0) {
@@ -115,15 +122,11 @@ class BgzfReader {
   }
   bool device_inflate_used() const { return device_batches_.load() != 0; }
   ~BgzfReader() {
-    if (producer_.joinable()) {
-      {
-        std::lock_guard<std::mutex> lk(mu_);
-        stop_ = true;
-      }
-      cv_.notify_all();
-      producer_.join();
-    }
+    stop_producer();
     if (f_) fclose(f_);
+    if (getenv("MPH_IO_TRACE"))  // measurement hook: what reading the file cost
+      fprintf(stderr, "[mph io] BGZF %s: %zu seeks, %zu compressed bytes read, %zu blocks inflated\n", path_.c_str(), seeks_,
+              size_t(cbytes_read_.load()), size_t(blocks_inflated_.load()));
   }
   BgzfReader(const BgzfReader&) = delete;
   BgzfReader& operator=(const BgzfReader&) = delete;
@@ -142,6 +145,36 @@ class BgzfReader {
     }
     pos_ = 0;
     return true;
+  }
+
+  // hands over everything inflated (the current block / batch) with its spans; the unread bytes start at `begin`
+  bool next_chunk(RawBytes& out, size_t& begin, std::vector<BgzfSpan>& spans) {
+    if (pos_ == block_.size() && !(threads_ > 1 ? next_batch() : next_block())) return false;
+    out.swap(block_);
+    spans.swap(spans_);
+    begin = pos_;
+    block_.clear();
+    spans_.clear();
+    pos_ = 0;
+    return true;
+  }
+
+  // Continues at a virtual offset (coff << 16 | offset inside the inflated block): drops the read-ahead, restarts the
+  // reading at the block's file offset and the inflated stream at the offset inside it.
+  void seek(uint64_t voff) {
+    stop_producer();
+    const uint64_t coff = voff >> 16;
+    if (coff >= file_bytes_ || fseeko(f_, off_t(coff), SEEK_SET) != 0) throw IoError("seek past the end of " + path_);
+    next_coff_ = seek_coff_ = coff;
+    ready_.clear();
+    stop_ = drained_ = false;
+    block_.clear();
+    spans_.clear();
+    pos_ = 0;
+    skip_ = size_t(voff & 0xFFFF);
+    skip_pending_ = true;
+    ++seeks_;
+    if (threads_ > 1) producer_ = std::thread([this] { produce(); });
   }
 
   // read exactly n bytes; returns false on clean EOF at a record boundary (0 bytes read)
@@ -165,8 +198,26 @@ class BgzfReader {
   }
 
  private:
+  void stop_producer() {
+    if (!producer_.joinable()) return;
+    {
+      std::lock_guard<std::mutex> lk(mu_);
+      stop_ = true;
+    }
+    cv_.notify_all();
+    producer_.join();
+  }
+  // the first block after a seek starts at the seek's in-block offset, which must lie inside it
+  void apply_skip() {
+    if (!skip_pending_) return;
+    skip_pending_ = false;
+    const size_t first_isize = spans_.size() > 1 ? size_t(spans_[1].ooff - spans_[0].ooff) : block_.size();
+    if (spans_.empty() || spans_[0].coff != seek_coff_ || skip_ > first_isize) throw IoError("virtual offset past the end of its BGZF block in " + path_);
+    pos_ = skip_;
+  }
   // reads one raw block (compressed payload appended to cbuf); false at end of file
-  bool read_raw(std::vector<uint8_t>& cbuf, Raw& r) {
+  bool read_raw(std::vector<uint8_t>& cbuf, Raw& r, uint64_t* coff = nullptr) {
+    if (coff) *coff = next_coff_;
     uint8_t hdr[18];
     size_t n = fread(hdr, 1, 18, f_);
     if (n == 0) return false;
@@ -191,10 +242,13 @@ class BgzfReader {
     uint32_t isize;
     memcpy(&isize, cbuf.data() + off + clen + 4, 4);
     r.coff = off; r.clen = clen; r.isize = isize; r.ooff = 0;
+    next_coff_ += uint64_t(bsize) + 1;
+    cbytes_read_ += uint64_t(bsize) + 1;
     return true;
   }
   void inflate_one(const uint8_t* in, size_t clen, uint8_t* out, size_t isize) const {
     if (isize == 0) return;
+    blocks_inflated_.fetch_add(1, std::memory_order_relaxed);
     if (fast_inflate_enabled().load(std::memory_order_relaxed)) {
       // the reader's own decoder (io/fast_inflate.hpp, ~1.3x zlib on BAM blocks); whatever it rejects goes through zlib below
       static thread_local std::unique_ptr<FastInflate> fast;
@@ -216,11 +270,14 @@ class BgzfReader {
     for (;;) {
       cbuf_.clear();
       Raw r;
-      if (!read_raw(cbuf_, r)) return false;
+      uint64_t coff;
+      if (!read_raw(cbuf_, r, &coff)) return false;
       block_.resize(r.isize);
+      spans_.assign(1, BgzfSpan{coff, 0});
       pos_ = 0;
-      if (r.isize == 0) continue;  // EOF marker / empty block
       inflate_one(cbuf_.data() + r.coff, r.clen, block_.data(), r.isize);
+      apply_skip();
+      if (pos_ == block_.size()) continue;  // EOF marker / empty block, or a seek to the end of a block
       return true;
     }
   }
@@ -228,6 +285,7 @@ class BgzfReader {
   // ---- threaded path: producer fills `ready_` (at most two batches ahead), consumer swaps them into block_
   struct Batch {
     RawBytes data;
+    std::vector<BgzfSpan> spans;
     bool eof = false;
     std::exception_ptr err;
   };
@@ -235,6 +293,7 @@ class BgzfReader {
   struct RawBatch {
     std::vector<uint8_t> cbuf;
     std::vector<Raw> raws;
+    std::vector<uint64_t> coffs;  // file offset of each block
     size_t total = 0;
     bool eof = false;
     std::exception_ptr err;
@@ -242,16 +301,19 @@ class BgzfReader {
   void read_raw_batch(RawBatch& rb) {
     rb.cbuf.clear();
     rb.raws.clear();
+    rb.coffs.clear();
     rb.total = 0;
     rb.eof = false;
     rb.err = nullptr;
     try {
       while (rb.raws.size() < batch_blocks_) {
         Raw r;
-        if (!read_raw(rb.cbuf, r)) { rb.eof = true; break; }
+        uint64_t coff;
+        if (!read_raw(rb.cbuf, r, &coff)) { rb.eof = true; break; }
         r.ooff = rb.total;
         rb.total += r.isize;
         rb.raws.push_back(r);
+        rb.coffs.push_back(coff);
       }
     } catch (...) {
       rb.err = std::current_exception();
@@ -264,8 +326,13 @@ class BgzfReader {
     RawBatch cur, nxt;
     read_raw_batch(cur);
     for (;;) {
+      {
+        std::lock_guard<std::mutex> lk(mu_);
+        if (stop_) return;
+      }
       Batch b;
       b.eof = cur.eof;
+      for (size_t i = 0; i < cur.raws.size(); ++i) b.spans.push_back(BgzfSpan{cur.coffs[i], int64_t(cur.raws[i].ooff)});
       bool have_next = false;
       try {
         b.data.resize(cur.total);
@@ -296,7 +363,7 @@ class BgzfReader {
           if (!cur.eof) { read_raw_batch(nxt); have_next = true; }
           helper.join();
           if (dev_err) inflater_ = nullptr;  // not available / failed: this batch and the rest go through zlib
-          else { on_device = true; device_batches_ += 1; }
+          else { on_device = true; device_batches_ += 1; blocks_inflated_ += cur.raws.size(); }
         }
         if (!on_device) {
           std::vector<std::thread> pool;
@@ -339,8 +406,10 @@ class BgzfReader {
       cv_.notify_all();
       if (b.err) std::rethrow_exception(b.err);
       block_ = std::move(b.data);
+      spans_ = std::move(b.spans);
       pos_ = 0;
-      if (!block_.empty()) return true;
+      if (!spans_.empty()) apply_skip();
+      if (pos_ < block_.size()) return true;
       if (drained_) return false;
     }
   }
@@ -349,7 +418,11 @@ class BgzfReader {
   FILE* f_ = nullptr;
   std::vector<uint8_t> cbuf_;
   RawBytes block_;
+  std::vector<BgzfSpan> spans_;  // of block_
   size_t pos_ = 0;
+  uint64_t next_coff_ = 0, seek_coff_ = 0;  // file offset of the next raw block / of the last seek
+  size_t skip_ = 0;
+  bool skip_pending_ = false;
   unsigned threads_ = 1;
   size_t file_bytes_ = 0;
   std::thread producer_;
@@ -358,8 +431,11 @@ class BgzfReader {
   std::deque<Batch> ready_;
   bool stop_ = false, drained_ = false;
   BatchInflater inflater_;
-  size_t batch_blocks_ = 256;
+  size_t batch_blocks_;
   std::atomic<size_t> device_batches_{0};
+  size_t seeks_ = 0;
+  std::atomic<uint64_t> cbytes_read_{0};
+  mutable std::atomic<uint64_t> blocks_inflated_{0};
 };
 
 // ---------------------------------------------------------------- BAM
@@ -460,8 +536,9 @@ struct BamFile {
   std::vector<int64_t> ref_lens;
   std::unordered_map<std::string, int> tid_of;
 
-  explicit BamFile(const std::string& path, unsigned inflate_threads = 1, BgzfReader::InflaterSpec inflater = BgzfReader::InflaterSpec())
-      : rd_(path, inflate_threads, std::move(inflater)) {
+  explicit BamFile(const std::string& path, unsigned inflate_threads = 1, BgzfReader::InflaterSpec inflater = BgzfReader::InflaterSpec(),
+                   size_t batch_blocks = 256)
+      : path_(path), rd_(path, inflate_threads, std::move(inflater), batch_blocks) {
     char magic[4];
     if (!rd_.read(magic, 4) || memcmp(magic, "BAM\1", 4) != 0) throw IoError("not a BAM file: " + path);
     auto must = [&](void* dst, size_t n) { if (!rd_.read(dst, n)) throw IoError("truncated BAM header: " + path); };
@@ -494,6 +571,10 @@ struct BamFile {
   // raw record stream after the header, in chunks (a record may straddle two chunks): for callers that frame and
   // parse the records themselves, in parallel
   bool next_chunk(RawBytes& out) { return rd_.next_chunk(out); }
+  // the same with where the bytes came from (virtual offsets), and a jump to a virtual offset: the indexed read buffer
+  bool next_chunk(RawBytes& out, size_t& begin, std::vector<BgzfSpan>& spans) { return rd_.next_chunk(out, begin, spans); }
+  void seek(uint64_t voff) { rd_.seek(voff); }
+  const std::string& path() const { return path_; }
 
   // next alignment record; false on EOF
   bool next(BamRecord& r) {
@@ -532,6 +613,7 @@ struct BamFile {
   }
 
  private:
+  std::string path_;
   BgzfReader rd_;
   std::vector<uint8_t> buf_;
 };
