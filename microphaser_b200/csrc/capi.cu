@@ -10,18 +10,20 @@
 #include <deque>
 #include <mutex>
 #include <unordered_map>
-#include <atomic>
 #include <chrono>
 #include <cstdarg>
 #include <fstream>
 #include <iostream>
 #include <memory>
+#include <optional>
 #include <thread>
+#include <utility>
 
 #include "../../include/microphaser_gpu.h"
 #include "host/cli.hpp"
 #include "host/peptides_host.hpp"
 #include "host/records_host.hpp"
+#include "host/shard_pipeline.hpp"
 #include "host/synth_files.hpp"
 #include "kernels/inflate_kernels.cuh"
 #include "kernels/peptide_kernels.cuh"
@@ -1498,148 +1500,17 @@ static void add_timing(mph_timing& a, const mph_timing& t) {
   a.n_records += t.n_records; a.kernel_launches += t.kernel_launches; a.n_replay_units += t.n_replay_units;
 }
 
-// Genes of an indexed BAM: this thread walks the GTF and fetches gene by gene in the reference's one-pass order
-// (reference slice, reads, variants), closing a shard every `reads_per_shard` reads (MPH_SHARD_READS overrides it). A pool
-// of workers packs each closed shard and phases it on whichever device is free; shards are written in order as they
-// complete. The walk waits while workers + 1 shards are fetched but not yet written, so the reads held in memory follow
-// the shard size, not the file size. A failure of the walk (a corrupt block late in the BAM) is reported after the
-// shards before it are written, as the reference, which streams, does.
-static void run_streamed(const std::vector<mph_ctx*>& ctxs, std::istream& gtf, mphio::BamFile& bam, const mphio::BamIndex& index,
-                         mphio::VcfFile& vcf, mphio::FastaIndexed& fasta, const IngestOptions& io, int fd_fa, int fd_tsv, int fd_n) {
-  const auto t_fetch0 = std::chrono::steady_clock::now();
-  std::vector<ParsedGene> parsed = read_gtf(gtf, io.mode);  // the unsorted-GTF panic comes before any output
-  const size_t n_dev = ctxs.size();
-  size_t per_dev = std::min<size_t>(12, std::max<size_t>(1, std::thread::hardware_concurrency() / n_dev));
-  if (const char* e = getenv("MPH_PACK_THREADS")) per_dev = size_t(std::max(1, atoi(e)));
-  uint64_t reads_per_shard = io.mode == 1 ? 2000000ull : 8000000ull;
-  if (const char* e = getenv("MPH_SHARD_READS")) reads_per_shard = uint64_t(std::max(1, atoi(e)));
-  const size_t n_workers = n_dev * per_dev;
-  std::mutex mu;
-  std::condition_variable cv;
-  std::deque<std::pair<size_t, std::vector<GeneInput>>> queue;  // closed shards waiting for a worker
-  std::map<size_t, mph_result*> results;                          // phased shards waiting for their turn to be written
-  size_t n_closed = 0, next_out = 0;
-  bool fetch_done = false;
-  int hw = 0;
-  std::exception_ptr first_err;
-  std::vector<std::mutex> dev_mu(n_dev);
-  std::vector<mph_timing> acc(n_dev, mph_timing{});
-  std::atomic<uint64_t> pack_us{0}, write_us{0};
-  auto worker = [&](size_t w) {
-    for (;;) {
-      std::pair<size_t, std::vector<GeneInput>> job;
-      {
-        std::unique_lock<std::mutex> lk(mu);
-        cv.wait(lk, [&] { return !queue.empty() || fetch_done; });
-        if (queue.empty()) return;
-        job = std::move(queue.front());
-        queue.pop_front();
-      }
-      const size_t k = job.first;
-      mph_result* res = nullptr;
-      std::exception_ptr err;
-      try {
-        bool skip;
-        {
-          std::lock_guard<std::mutex> lk(mu);
-          skip = first_err != nullptr;
-        }
-        if (!skip) {
-          const auto tp0 = std::chrono::steady_clock::now();
-          Packer packer(io.window_len, io.mode);
-          pack_genes(job.second, 0, job.second.size(), packer);
-          std::vector<GeneInput>().swap(job.second);  // the reads' batches are free once packed
-          std::unique_ptr<mph_batch> batch(new mph_batch);
-          batch->b = std::move(packer.batch());
-          finish_batch(batch.get(), false);
-          pack_us += uint64_t(std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now() - tp0).count());
-          // a context is not re-entrant: the first free device, else this worker's own
-          size_t dv = n_dev;
-          for (size_t d = 0; d < n_dev && dv == n_dev; ++d)
-            if (dev_mu[d].try_lock()) dv = d;
-          if (dv == n_dev) {
-            dv = w % n_dev;
-            dev_mu[dv].lock();
-          }
-          std::lock_guard<std::mutex> dl(dev_mu[dv], std::adopt_lock);
-          phase_batch_impl(ctxs[dv], batch.get(), &res);
-          add_timing(acc[dv], ctxs[dv]->timing);
-        }
-      } catch (...) {
-        err = std::current_exception();
-      }
-      // ordered concatenation: shard k goes out when shards 0 .. k-1 are out; after a failure nothing later is written
-      std::lock_guard<std::mutex> lk(mu);
-      if (err && !first_err) first_err = err;
-      results[k] = res;
-      for (auto it = results.find(next_out); it != results.end(); it = results.find(next_out)) {
-        if (it->second) {
-          const auto tw0 = std::chrono::steady_clock::now();
-          if (!first_err && mph_result_write(it->second, fd_fa, fd_tsv, fd_n, &hw) != MPH_OK && !first_err)
-            first_err = std::make_exception_ptr(std::runtime_error(g_last_error));
-          write_us += uint64_t(std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now() - tw0).count());
-          delete it->second;
-        }
-        results.erase(it);
-        ++next_out;
-      }
-      cv.notify_all();
-    }
-  };
-  std::vector<std::thread> pool;
-  for (size_t w = 0; w < n_workers; ++w) pool.emplace_back(worker, w);
-  std::exception_ptr fetch_err;
-  try {
-    ReadBuffer reads(bam, index);
-    VariantBuffer variants(vcf);
-    std::vector<GeneInput> shard;
-    uint64_t shard_reads = 0;
-    auto close_shard = [&] {
-      std::unique_lock<std::mutex> lk(mu);
-      cv.wait(lk, [&] { return n_closed - next_out < n_workers + 1 || first_err; });
-      queue.emplace_back(n_closed++, std::move(shard));
-      shard.clear();
-      shard_reads = 0;
-      cv.notify_all();
-    };
-    try {
-      for (ParsedGene& pg : parsed) {
-        if (pg.biotype != "protein_coding") continue;  // :1964
-        {
-          std::lock_guard<std::mutex> lk(mu);
-          if (first_err) break;
-        }
-        shard.push_back(fetch_gene(std::move(pg.gene), reads, variants, vcf, fasta, io));
-        shard_reads += shard.back().n_reads;
-        if (shard_reads >= reads_per_shard) close_shard();
-      }
-    } catch (...) {
-      fetch_err = std::current_exception();  // the genes fetched before the failure are still phased and written
-    }
-    if (!shard.empty()) close_shard();
-  } catch (...) {
-    if (!fetch_err) fetch_err = std::current_exception();
-  }
-  const double fetch_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_fetch0).count();
-  {
-    std::lock_guard<std::mutex> lk(mu);
-    fetch_done = true;
-  }
-  cv.notify_all();
-  for (auto& t : pool) t.join();
-  for (auto& kv : results) delete kv.second;
-  for (size_t dv = 0; dv < n_dev; ++dv) ctxs[dv]->timing = acc[dv];
-  ctxs[0]->timing.ingest_ms = fetch_ms;
-  ctxs[0]->timing.pack_ms = double(pack_us.load()) / 1000.0;
-  ctxs[0]->timing.write_ms = double(write_us.load()) / 1000.0;
-  if (first_err) std::rethrow_exception(first_err);
-  if (fetch_err) std::rethrow_exception(fetch_err);
-}
+using FilePipeline = ShardPipeline<std::vector<GeneInput>, std::unique_ptr<mph_batch>, std::unique_ptr<mph_result>, mph_timing>;
 
-// shared by the single- and multi-device file drivers
-static void run_somatic_files(const std::vector<mph_ctx*>& ctxs, const char* bam_path, const char* ref_path, const char* variants_path,
-                              const char* gtf_path, const char* fasta_out_path, const char* tsv_path, const char* normal_path,
-                              uint32_t window_len, int warn_only, int mode = 0) {
+// The file driver of the single- and multi-device entry points. Without an index the whole BAM is loaded and the genes
+// are cut into balanced shards, a fixed run of consecutive shards per device. With an index next to the BAM this thread
+// fetches the genes one by one in the reference's one-pass order (reference slice, reads, variants) and closes a shard
+// every `reads_per_shard` reads for whichever device is free; it waits while workers + 1 shards are not yet written, so
+// the reads held in memory follow the shard size, not the file size, and a failure of the walk (a corrupt block late in
+// the BAM) is reported after the shards before it are written, as the reference, which streams, does.
+static void run_files(const std::vector<mph_ctx*>& ctxs, const char* bam_path, const char* ref_path, const char* variants_path,
+                      const char* gtf_path, const char* fasta_out_path, const char* tsv_path, const char* normal_path,
+                      uint32_t window_len, int warn_only, int mode) {
   // BGZF inflate of the alignment file runs on a few host threads (MPH_IO_THREADS, default min(cores, 8))
   // BGZF inflate is the largest single host cost of the file driver (about 0.7 core-seconds per million 150 bp reads with zlib):
   // every core takes blocks
@@ -1703,107 +1574,90 @@ static void run_somatic_files(const std::vector<mph_ctx*>& ctxs, const char* bam
       if (!gf) throw std::runtime_error(std::string("cannot open ") + gtf_path);
       gin = &gf;
     }
-    if (index) {
-      run_streamed(ctxs, *gin, bam, *index, vcf, fasta, io, fd_fa, fd_tsv, fd_n);
-      if (gpu_inflate && getenv("MPH_IO_TRACE"))
-        fprintf(stderr, "[mph io] device inflate: %zu batches, %.1f MB in, %.1f MB out, %.1f ms inside the inflater (copies + kernel)%s\n", gpu_inflate->batches,
-                gpu_inflate->bytes_in / 1e6, gpu_inflate->bytes_out / 1e6, gpu_inflate->ms_total, bam.device_inflate_used() ? "" : " - not used (small file or fallback to zlib)");
-      close_all();
-      return;
-    }
+    const size_t n_dev = ctxs.size();
+    auto pack = [&](std::vector<GeneInput>& genes) {
+      Packer packer(window_len, mode);
+      pack_genes(genes, 0, genes.size(), packer);
+      std::unique_ptr<mph_batch> batch(new mph_batch);
+      batch->b = std::move(packer.batch());
+      finish_batch(batch.get(), false);
+      return batch;
+    };
+    auto phase = [&](size_t dv, std::unique_ptr<mph_batch>& batch, mph_timing& sum) {
+      mph_result* res = nullptr;
+      phase_batch_impl(ctxs[dv], batch.get(), &res);
+      add_timing(sum, ctxs[dv]->timing);  // a device's timing is the sum over its shards
+      return std::unique_ptr<mph_result>(res);
+    };
+    int hw = 0;  // the TSV header goes out with the first row only
+    auto write = [&](std::unique_ptr<mph_result>& res) {
+      if (mph_result_write(res.get(), fd_fa, fd_tsv, fd_n, &hw) != MPH_OK) throw std::runtime_error(g_last_error);
+    };
+    std::unique_ptr<ReadBufferLoader> loader;  // whole file: holds the reads the genes point into, so it outlives the pipeline
+    std::optional<FilePipeline> pipe;
+    std::exception_ptr err;  // a failure of the indexed walk; a failure in the pipeline replaces it, being reported first
+    // packing threads per device: one per core up to 12, MPH_PACK_THREADS overrides it
+    const size_t cores_per_dev = std::min<size_t>(12, std::max<size_t>(1, std::thread::hardware_concurrency() / n_dev));
+    const char* pack_threads = getenv("MPH_PACK_THREADS");
+    uint64_t reads_per_shard = mode == 1 ? 2000000ull : 8000000ull;
     const auto t_ingest0 = std::chrono::steady_clock::now();
-    ReadBufferLoader loader(bam);  // the BAM loads on its own thread while this one parses the GTF and fetches reference slices and variants
-    std::vector<GeneInput> genes = ingest_genes_with(*gin, [&]() -> ReadBuffer& { return loader.get(); }, vcf, fasta, io, true);
-    const double ingest_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_ingest0).count();
+    double ingest_ms;
+    if (index) {
+      std::vector<ParsedGene> parsed = read_gtf(*gin, mode);  // the unsorted-GTF panic comes before any output
+      if (const char* e = getenv("MPH_SHARD_READS")) reads_per_shard = uint64_t(std::max(1, atoi(e)));
+      const size_t n_workers = n_dev * (pack_threads ? size_t(std::max(1, atoi(pack_threads))) : cores_per_dev);
+      pipe.emplace(n_dev, n_workers, n_workers + 1, pack, phase, write);
+      std::vector<GeneInput> shard;
+      uint64_t shard_reads = 0;
+      try {
+        walk_indexed_genes(std::move(parsed), bam, *index, vcf, fasta, io, [&](GeneInput&& gi) {
+          shard_reads += gi.n_reads;
+          shard.push_back(std::move(gi));
+          if (shard_reads < reads_per_shard) return !pipe->failed();
+          shard_reads = 0;
+          return pipe->submit(std::exchange(shard, {}), FilePipeline::kAnyDevice);
+        });
+      } catch (...) {
+        err = std::current_exception();  // the genes fetched before the failure are still phased and written
+      }
+      if (!shard.empty()) pipe->submit(std::move(shard), FilePipeline::kAnyDevice);
+      ingest_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_ingest0).count();
+    } else {
+      loader.reset(new ReadBufferLoader(bam));  // the BAM loads on its own thread while this one parses the GTF and fetches reference slices and variants
+      std::vector<GeneInput> genes = ingest_genes_with(*gin, [&]() -> ReadBuffer& { return loader->get(); }, vcf, fasta, io, true);
+      ingest_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_ingest0).count();
+      // one contiguous gene range per device, no exchange between shards (SURVEY.md §8(e)); a device's range is cut
+      // further so that several host threads pack in parallel, while its phase calls run one after the other
+      uint64_t total_reads = 0;
+      for (auto& g : genes) total_reads += g.n_reads;
+      const size_t per_dev = pack_threads ? size_t(std::max(1, atoi(pack_threads))) : total_reads > 200000 * n_dev ? cores_per_dev : 1;
+      // more shards than packing threads when the input is large: a shard's records are written and freed as soon as all
+      // earlier shards are out, which bounds the memory held in records (the normal mode writes one per window)
+      size_t n_shards = std::max<size_t>(n_dev * per_dev, size_t((total_reads + reads_per_shard - 1) / reads_per_shard));
+      n_shards = (n_shards + n_dev - 1) / n_dev * n_dev;  // the same number of consecutive shards per device
+      const size_t shards_per_dev = n_shards / n_dev;
+      const std::vector<size_t> cut = partition_genes(genes, n_shards);
+      pipe.emplace(n_dev, std::min(n_shards, n_dev * per_dev), 0, pack, phase, write);
+      for (size_t k = 0; k < n_shards; ++k) {
+        std::vector<GeneInput> shard(std::make_move_iterator(genes.begin() + cut[k]), std::make_move_iterator(genes.begin() + cut[k + 1]));
+        if (!pipe->submit(std::move(shard), k / shards_per_dev)) break;
+      }
+    }
+    FilePipeline::Totals totals;
+    try {
+      pipe->finish(totals);
+    } catch (...) {
+      err = std::current_exception();
+    }
+    for (size_t dv = 0; dv < n_dev; ++dv) ctxs[dv]->timing = totals.per_dev[dv];
+    // host stages of the file driver (the first context carries them)
+    ctxs[0]->timing.ingest_ms = ingest_ms;
+    ctxs[0]->timing.pack_ms = double(totals.pack_us) / 1000.0;
+    ctxs[0]->timing.write_ms = double(totals.write_us) / 1000.0;
+    if (err) std::rethrow_exception(err);
     if (gpu_inflate && getenv("MPH_IO_TRACE"))
       fprintf(stderr, "[mph io] device inflate: %zu batches, %.1f MB in, %.1f MB out, %.1f ms inside the inflater (copies + kernel)%s\n", gpu_inflate->batches,
               gpu_inflate->bytes_in / 1e6, gpu_inflate->bytes_out / 1e6, gpu_inflate->ms_total, bam.device_inflate_used() ? "" : " - not used (small file or fallback to zlib)");
-    std::atomic<uint64_t> pack_us{0}, write_us{0};
-    // one contiguous gene range per device, no exchange between shards (SURVEY.md §8(e)); a device's range is cut
-    // further so that several host threads pack in parallel, while its phase calls run one after the other
-    const size_t n_dev = ctxs.size();
-    uint64_t total_reads = 0;
-    for (auto& g : genes) total_reads += g.n_reads;
-    size_t per_dev = 1;
-    if (total_reads > 200000 * n_dev)
-      per_dev = std::min<size_t>(12, std::max<size_t>(1, std::thread::hardware_concurrency() / n_dev));
-    if (const char* e = getenv("MPH_PACK_THREADS")) per_dev = size_t(std::max(1, atoi(e)));
-    // more shards than packing threads when the input is large: a shard's records are written and freed as soon as all
-    // earlier shards are out, which bounds the memory held in records (the normal mode writes one per window)
-    const uint64_t reads_per_shard = mode == 1 ? 2000000ull : 8000000ull;
-    size_t n_shards = std::max<size_t>(n_dev * per_dev, size_t((total_reads + reads_per_shard - 1) / reads_per_shard));
-    n_shards = (n_shards + n_dev - 1) / n_dev * n_dev;  // the same number of consecutive shards per device
-    const size_t shards_per_dev = n_shards / n_dev;
-    const std::vector<size_t> cut = partition_genes(genes, n_shards);
-    std::vector<mph_result*> results(n_shards, nullptr);
-    std::vector<uint8_t> done(n_shards, 0);
-    std::vector<std::mutex> dev_mu(n_dev);
-    std::mutex out_mu;
-    size_t next_out = 0;
-    int hw = 0;
-    std::exception_ptr first_err;
-    std::vector<mph_timing> acc(n_dev, mph_timing{});  // a device's timing is the sum over its shards
-    // ordered concatenation: shard k goes out when shards 0 .. k-1 are out; the TSV header goes out with the first row only.
-    // After a failure nothing later than the failing shard is written (the reference stops at that point, too).
-    auto shard_finished = [&](size_t k, std::exception_ptr err) {
-      std::lock_guard<std::mutex> lk(out_mu);
-      done[k] = 1;
-      if (err && !first_err) first_err = err;
-      while (next_out < n_shards && done[next_out]) {
-        if (results[next_out]) {
-          const auto tw0 = std::chrono::steady_clock::now();
-          if (!first_err && mph_result_write(results[next_out], fd_fa, fd_tsv, fd_n, &hw) != MPH_OK && !first_err)
-            first_err = std::make_exception_ptr(std::runtime_error(g_last_error));
-          write_us += uint64_t(std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now() - tw0).count());
-          delete results[next_out];
-          results[next_out] = nullptr;
-        }
-        ++next_out;
-      }
-    };
-    std::atomic<size_t> next_shard{0};
-    auto worker = [&] {
-      for (;;) {
-        const size_t k = next_shard.fetch_add(1);
-        if (k >= n_shards) return;
-        std::exception_ptr err;
-        try {
-          {
-            std::lock_guard<std::mutex> lk(out_mu);
-            if (first_err) { done[k] = 1; continue; }
-          }
-          const auto tp0 = std::chrono::steady_clock::now();
-          Packer packer(window_len, mode);
-          pack_genes(genes, cut[k], cut[k + 1], packer);
-          std::unique_ptr<mph_batch> batch(new mph_batch);
-          batch->b = std::move(packer.batch());
-          finish_batch(batch.get(), false);
-          pack_us += uint64_t(std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now() - tp0).count());
-          const size_t dv = k / shards_per_dev;
-          std::lock_guard<std::mutex> lk(dev_mu[dv]);  // a context is not re-entrant
-          phase_batch_impl(ctxs[dv], batch.get(), &results[k]);
-          add_timing(acc[dv], ctxs[dv]->timing);
-        } catch (...) {
-          err = std::current_exception();
-        }
-        shard_finished(k, err);
-      }
-    };
-    const size_t n_workers = std::min(n_shards, n_dev * per_dev);
-    if (n_workers == 1) {
-      worker();
-    } else {
-      std::vector<std::thread> th;
-      for (size_t w = 0; w < n_workers; ++w) th.emplace_back(worker);
-      for (auto& t : th) t.join();
-    }
-    for (size_t dv = 0; dv < n_dev; ++dv) ctxs[dv]->timing = acc[dv];
-    // host stages of the file driver (the first context carries them)
-    ctxs[0]->timing.ingest_ms = ingest_ms;
-    ctxs[0]->timing.pack_ms = double(pack_us.load()) / 1000.0;
-    ctxs[0]->timing.write_ms = double(write_us.load()) / 1000.0;
-    for (auto r : results) delete r;
-    if (first_err) std::rethrow_exception(first_err);
   } catch (...) {
     close_all();
     throw;
@@ -1811,46 +1665,43 @@ static void run_somatic_files(const std::vector<mph_ctx*>& ctxs, const char* bam
   close_all();
 }
 
+// What the mph_run_* file entry points share: a null argument is reported on `null_ctx`, a window length the packer
+// cannot take and the run's own errors on the first context. Only the normal mode (mode 1) has no `normal_path`.
+static int run_files_checked(mph_ctx* null_ctx, mph_ctx* const* ctxs, int n_ctx, const char* bam_path, const char* ref_path,
+                             const char* variants_path, const char* gtf_path, const char* fasta_out_path, const char* tsv_path,
+                             const char* normal_path, uint32_t window_len, int warn_only, int mode) {
+  if (!ctxs || n_ctx < 1 || !bam_path || !ref_path || !variants_path || !gtf_path || !fasta_out_path || !tsv_path || (mode == 0 && !normal_path))
+    return fail(null_ctx, MPH_ERR_INPUT, "null argument");
+  if (window_len == 0 || window_len % 3 != 0) return fail(ctxs[0], MPH_ERR_UNSUPPORTED, "window length must be a positive multiple of 3");
+  return guarded(ctxs[0], [&] {
+    run_files(std::vector<mph_ctx*>(ctxs, ctxs + n_ctx), bam_path, ref_path, variants_path, gtf_path, fasta_out_path, tsv_path, normal_path,
+              window_len, warn_only, mode);
+  });
+}
+
 int mph_run_somatic(mph_ctx* ctx, const char* bam_path, const char* ref_path, const char* variants_path, const char* gtf_path,
                     const char* fasta_out_path, const char* tsv_path, const char* normal_path, uint32_t window_len, int warn_only) {
-  if (!ctx || !bam_path || !ref_path || !variants_path || !gtf_path || !fasta_out_path || !tsv_path || !normal_path)
-    return fail(ctx, MPH_ERR_INPUT, "null argument");
-  if (window_len == 0 || window_len % 3 != 0) return fail(ctx, MPH_ERR_UNSUPPORTED, "window length must be a positive multiple of 3");
-  return guarded(ctx, [&] {
-    run_somatic_files({ctx}, bam_path, ref_path, variants_path, gtf_path, fasta_out_path, tsv_path, normal_path, window_len, warn_only);
-  });
+  if (!ctx) return fail(nullptr, MPH_ERR_INPUT, "null argument");
+  return run_files_checked(ctx, &ctx, 1, bam_path, ref_path, variants_path, gtf_path, fasta_out_path, tsv_path, normal_path, window_len, warn_only, 0);
 }
 
 int mph_run_normal(mph_ctx* ctx, const char* bam_path, const char* ref_path, const char* variants_path, const char* gtf_path,
                    const char* fasta_out_path, const char* tsv_path, uint32_t window_len, int warn_only) {
-  if (!ctx || !bam_path || !ref_path || !variants_path || !gtf_path || !fasta_out_path || !tsv_path) return fail(ctx, MPH_ERR_INPUT, "null argument");
-  if (window_len == 0 || window_len % 3 != 0) return fail(ctx, MPH_ERR_UNSUPPORTED, "window length must be a positive multiple of 3");
-  return guarded(ctx, [&] {
-    run_somatic_files({ctx}, bam_path, ref_path, variants_path, gtf_path, fasta_out_path, tsv_path, nullptr, window_len, warn_only, 1);
-  });
+  if (!ctx) return fail(nullptr, MPH_ERR_INPUT, "null argument");
+  return run_files_checked(ctx, &ctx, 1, bam_path, ref_path, variants_path, gtf_path, fasta_out_path, tsv_path, nullptr, window_len, warn_only, 1);
 }
 
 int mph_run_somatic_multi(mph_ctx* const* ctxs, int n_ctx, const char* bam_path, const char* ref_path, const char* variants_path,
                           const char* gtf_path, const char* fasta_out_path, const char* tsv_path, const char* normal_path,
                           uint32_t window_len, int warn_only) {
-  if (!ctxs || n_ctx < 1 || !bam_path || !ref_path || !variants_path || !gtf_path || !fasta_out_path || !tsv_path || !normal_path)
-    return fail(nullptr, MPH_ERR_INPUT, "null argument");
-  if (window_len == 0 || window_len % 3 != 0) return fail(ctxs[0], MPH_ERR_UNSUPPORTED, "window length must be a positive multiple of 3");
-  return guarded(ctxs[0], [&] {
-    run_somatic_files(std::vector<mph_ctx*>(ctxs, ctxs + n_ctx), bam_path, ref_path, variants_path, gtf_path, fasta_out_path, tsv_path,
-                      normal_path, window_len, warn_only);
-  });
+  return run_files_checked(nullptr, ctxs, n_ctx, bam_path, ref_path, variants_path, gtf_path, fasta_out_path, tsv_path, normal_path, window_len,
+                           warn_only, 0);
 }
 
 int mph_run_normal_multi(mph_ctx* const* ctxs, int n_ctx, const char* bam_path, const char* ref_path, const char* variants_path,
                          const char* gtf_path, const char* fasta_out_path, const char* tsv_path, uint32_t window_len, int warn_only) {
-  if (!ctxs || n_ctx < 1 || !bam_path || !ref_path || !variants_path || !gtf_path || !fasta_out_path || !tsv_path)
-    return fail(nullptr, MPH_ERR_INPUT, "null argument");
-  if (window_len == 0 || window_len % 3 != 0) return fail(ctxs[0], MPH_ERR_UNSUPPORTED, "window length must be a positive multiple of 3");
-  return guarded(ctxs[0], [&] {
-    run_somatic_files(std::vector<mph_ctx*>(ctxs, ctxs + n_ctx), bam_path, ref_path, variants_path, gtf_path, fasta_out_path, tsv_path,
-                      nullptr, window_len, warn_only, 1);
-  });
+  return run_files_checked(nullptr, ctxs, n_ctx, bam_path, ref_path, variants_path, gtf_path, fasta_out_path, tsv_path, nullptr, window_len,
+                           warn_only, 1);
 }
 
 int mph_translate(mph_ctx* ctx, const uint8_t* nt, const uint64_t* off, const int8_t* frame, uint64_t n, uint8_t* aa, const uint64_t* aa_off,

@@ -42,10 +42,11 @@ bool parse_args(int argc, char** argv, const std::vector<Spec>& specs, std::map<
   return true;
 }
 
-int finish(mph_ctx* ctx, int rc) {
+// exit status of a run; `unsupported` leads the message of MPH_ERR_UNSUPPORTED
+int finish(mph_ctx* ctx, int rc, const char* unsupported) {
   int status = 0;
   if (rc == MPH_ERR_PANIC) { fprintf(stderr, "thread 'main' panicked at '%s'\n", mph_last_error(ctx)); status = 101; }
-  else if (rc == MPH_ERR_UNSUPPORTED) { fprintf(stderr, "microphaser: not supported by the GPU path: %s\n", mph_last_error(ctx)); status = 3; }
+  else if (rc == MPH_ERR_UNSUPPORTED) { fprintf(stderr, "microphaser: %s: %s\n", unsupported, mph_last_error(ctx)); status = 3; }
   else if (rc != MPH_OK) { fprintf(stderr, "%s\n", mph_last_error(ctx)); status = 1; }
   return status;
 }
@@ -54,27 +55,24 @@ int finish(mph_ctx* ctx, int rc) {
 int run_secondary(const std::string& sub, int argc, char** argv) {
   std::map<std::string, std::string> opt;
   std::vector<std::string> pos;
-  mph_ctx* ctx = nullptr;
-  if (sub == "filter") {
+  const bool filter = sub == "filter";
+  if (filter) {
     if (!parse_args(argc, argv, {{"tsv", 't', true}, {"reference", 'r', true}, {"tsv-output", 'o', true}, {"similar-removed", 's', true},
                                  {"removed-peptides", 'p', true}, {"normal-output", 'n', true}, {"peptide-length", 'l', true}, {"verbose", 'v', false}}, opt, pos)) return 1;
     if (!opt.count("tsv") || !opt.count("reference")) { fprintf(stderr, "error: The following required arguments were not provided: --tsv <FILE> --reference <FILE>\n"); return 1; }
-    auto get = [&](const char* k, const char* d) { return opt.count(k) ? opt[k] : std::string(d); };
-    const uint32_t l = uint32_t(strtoul(get("peptide-length", "9").c_str(), nullptr, 10));
-    if (mph_ctx_create(getenv("MPH_DEVICE") ? atoi(getenv("MPH_DEVICE")) : 0, &ctx) != MPH_OK) { fprintf(stderr, "microphaser: %s\n", mph_last_error(nullptr)); return 1; }
-    const int rc = mph_run_filter(ctx, opt["reference"].c_str(), opt["tsv"].c_str(), "-", get("normal-output", "normal.filtered.fa").c_str(),
-                                  get("tsv-output", "info.filtered.tsv").c_str(), get("similar-removed", "info.removed.tsv").c_str(),
-                                  get("removed-peptides", "peptides.removed.fasta").c_str(), l);
-    const int st = finish(ctx, rc);
-    mph_ctx_destroy(ctx);
-    return st;
+  } else {
+    if (!parse_args(argc, argv, {{"reference", 'r', true}, {"output", 'o', true}, {"peptide-length", 'l', true}, {"verbose", 'v', false}}, opt, pos)) return 1;
+    if (!opt.count("reference") || !opt.count("output")) { fprintf(stderr, "error: The following required arguments were not provided: --reference <FILE> --output <FILE>\n"); return 1; }
   }
-  if (!parse_args(argc, argv, {{"reference", 'r', true}, {"output", 'o', true}, {"peptide-length", 'l', true}, {"verbose", 'v', false}}, opt, pos)) return 1;
-  if (!opt.count("reference") || !opt.count("output")) { fprintf(stderr, "error: The following required arguments were not provided: --reference <FILE> --output <FILE>\n"); return 1; }
-  const uint32_t l = opt.count("peptide-length") ? uint32_t(strtoul(opt["peptide-length"].c_str(), nullptr, 10)) : 9;
+  auto get = [&](const char* k, const char* d) { return opt.count(k) ? opt[k] : std::string(d); };
+  const uint32_t l = uint32_t(strtoul(get("peptide-length", "9").c_str(), nullptr, 10));
+  mph_ctx* ctx = nullptr;
   if (mph_ctx_create(getenv("MPH_DEVICE") ? atoi(getenv("MPH_DEVICE")) : 0, &ctx) != MPH_OK) { fprintf(stderr, "microphaser: %s\n", mph_last_error(nullptr)); return 1; }
-  const int rc = mph_run_build_reference(ctx, opt["reference"].c_str(), opt["output"].c_str(), "-", l);
-  const int st = finish(ctx, rc);
+  const int rc = filter ? mph_run_filter(ctx, opt["reference"].c_str(), opt["tsv"].c_str(), "-", get("normal-output", "normal.filtered.fa").c_str(),
+                                         get("tsv-output", "info.filtered.tsv").c_str(), get("similar-removed", "info.removed.tsv").c_str(),
+                                         get("removed-peptides", "peptides.removed.fasta").c_str(), l)
+                        : mph_run_build_reference(ctx, opt["reference"].c_str(), opt["output"].c_str(), "-", l);
+  const int st = finish(ctx, rc, "not supported by the GPU path");
   mph_ctx_destroy(ctx);
   return st;
 }
@@ -92,29 +90,9 @@ int main(int argc, char** argv) {
   }
   std::map<std::string, std::string> opt;
   std::vector<std::string> pos;
-  bool warn_only = false;
-  const Spec specs[] = {{"ref", 'r', true}, {"variants", 'b', true}, {"window-len", 'w', true}, {"tsv", 't', true},
-                        {"normal-output", 'n', true}, {"unsupported-allele-warning-only", 'u', false}, {"verbose", 'v', false}};
-  for (int i = 2; i < argc; ++i) {
-    std::string s = argv[i];
-    const Spec* sp = nullptr;
-    std::string val;
-    bool have = false;
-    if (s.rfind("--", 0) == 0) {
-      std::string name = s.substr(2);
-      size_t eq = name.find('=');
-      if (eq != std::string::npos) { val = name.substr(eq + 1); name = name.substr(0, eq); have = true; }
-      for (auto& x : specs) if (name == x.lng) sp = &x;
-    } else if (s.size() >= 2 && s[0] == '-') {
-      for (auto& x : specs) if (s[1] == x.shrt) sp = &x;
-      if (sp && s.size() > 2) { val = s.substr(s[2] == '=' ? 3 : 2); have = true; }
-    } else { pos.push_back(s); continue; }
-    if (!sp) { fprintf(stderr, "error: Found argument '%s' which wasn't expected\n", s.c_str()); return 1; }
-    if (sp->value) {
-      if (!have) { if (i + 1 >= argc) { fprintf(stderr, "error: The argument '--%s' requires a value\n", sp->lng); return 1; } val = argv[++i]; }
-      opt[sp->lng] = val;
-    } else if (std::string(sp->lng) == "unsupported-allele-warning-only") warn_only = true;
-  }
+  if (!parse_args(argc, argv, {{"ref", 'r', true}, {"variants", 'b', true}, {"window-len", 'w', true}, {"tsv", 't', true}, {"normal-output", 'n', true},
+                               {"unsupported-allele-warning-only", 'u', false}, {"verbose", 'v', false}}, opt, pos)) return 1;
+  const bool warn_only = opt.count("unsupported-allele-warning-only") != 0;
   if (pos.size() != 1 || !opt.count("ref") || !opt.count("variants")) {
     fprintf(stderr, "error: The following required arguments were not provided: <tumor-sample> --ref <FILE> --variants <FILE>\n");
     return 1;
@@ -146,10 +124,7 @@ int main(int argc, char** argv) {
   else
     rc = mph_run_somatic_multi(ctxs.data(), int(ctxs.size()), pos[0].c_str(), opt["ref"].c_str(), opt["variants"].c_str(), "-", "-", tsv.c_str(),
                                nrm.c_str(), wl, warn_only);
-  int status = 0;
-  if (rc == MPH_ERR_PANIC) { fprintf(stderr, "thread 'main' panicked at '%s'\n", mph_last_error(ctx)); status = 101; }
-  else if (rc == MPH_ERR_UNSUPPORTED) { fprintf(stderr, "microphaser: input needs the serial replay path, which is not implemented: %s\n", mph_last_error(ctx)); status = 3; }
-  else if (rc != MPH_OK) { fprintf(stderr, "%s\n", mph_last_error(ctx)); status = 1; }
+  const int status = finish(ctx, rc, "input needs the serial replay path, which is not implemented");
   for (auto c : ctxs) mph_ctx_destroy(c);
   return status;
 }

@@ -1108,6 +1108,19 @@ inline void pack_genes(std::vector<GeneInput>& genes, size_t lo, size_t hi, Pack
   }
 }
 
+// The protein-coding genes of a parsed GTF, fetched one by one through the BAM index in GTF order and handed to
+// `on_gene(GeneInput&&)`; the walk stops when that returns false.
+template <class OnGene>
+inline void walk_indexed_genes(std::vector<ParsedGene> genes, mphio::BamFile& bam, const mphio::BamIndex& index, mphio::VcfFile& vcf,
+                               mphio::FastaIndexed& fasta, const IngestOptions& opt, OnGene&& on_gene) {
+  ReadBuffer reads(bam, index);
+  VariantBuffer variants(vcf);
+  for (ParsedGene& pg : genes) {
+    if (pg.biotype != "protein_coding") continue;  // :1964
+    if (!on_gene(fetch_gene(std::move(pg.gene), reads, variants, vcf, fasta, opt))) return;
+  }
+}
+
 // Builds the batch for every protein-coding gene of the GTF, in GTF order. With an index next to the BAM the reads are
 // fetched through it gene by gene; without one the whole file is loaded first.
 inline void ingest(std::istream& gtf, mphio::BamFile& bam, mphio::VcfFile& vcf, mphio::FastaIndexed& fasta, const IngestOptions& opt,
@@ -1115,14 +1128,12 @@ inline void ingest(std::istream& gtf, mphio::BamFile& bam, mphio::VcfFile& vcf, 
   const std::string bai = mphio::BamIndex::locate(bam.path());
   if (!bai.empty()) {
     const mphio::BamIndex index(bai, bam.ref_names.size(), bam.file_bytes());
-    ReadBuffer reads(bam, index);
-    VariantBuffer variants(vcf);
     std::vector<GeneInput> one(1);
-    for (ParsedGene& pg : read_gtf(gtf, opt.mode)) {
-      if (pg.biotype != "protein_coding") continue;  // :1964
-      one[0] = fetch_gene(std::move(pg.gene), reads, variants, vcf, fasta, opt);
+    walk_indexed_genes(read_gtf(gtf, opt.mode), bam, index, vcf, fasta, opt, [&](GeneInput&& gi) {
+      one[0] = std::move(gi);
       pack_genes(one, 0, 1, packer);
-    }
+      return true;
+    });
     return;
   }
   ReadBufferLoader loader(bam);
