@@ -43,6 +43,7 @@ def build_all(force=False, verbose=False):
         for src in (os.path.join(CSRC, "kernels", "phase_kernels.cu"), os.path.join(CSRC, "kernels", "replay_kernels.cu"),
                     os.path.join(CSRC, "kernels", "normal_kernels.cu"), os.path.join(CSRC, "kernels", "peptide_kernels.cu"),
                     os.path.join(CSRC, "kernels", "record_kernels.cu"), os.path.join(CSRC, "kernels", "inflate_kernels.cu"),
+                    os.path.join(CSRC, "kernels", "block_kernels.cu"),
                     os.path.join(CSRC, "capi.cu")):
             obj = os.path.join(OUT, os.path.basename(src) + ".o")
             cmd = [NVCC] + NVFLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-c", src, "-o", obj]

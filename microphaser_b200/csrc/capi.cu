@@ -223,7 +223,8 @@ struct mph_ctx {
   DevBuf<int> win_diff;
   DevBuf<uint64_t> call_S, call_B;
   DevBuf<MphWinOut> win_out, iw_out;
-  DevBuf<MphHist> hist;
+  DevBuf<MphHist> hist, spill;
+  DevBuf<MphSpillWin> spq, spq_rp;
   DevBuf<MphHap> hap0, hapx, iw_hap0;
   DevBuf<unsigned long long> sums, win_id;
   mph_timing timing = {};
@@ -365,6 +366,8 @@ void prepare(mph_ctx* c, const mph_batch* mb) {
   c->win_out.ensure(nw + 1); c->hap0.ensure(nw + 1); c->win_flag.ensure(nw + 1);
   c->block_counts.ensure(nw / 1024 + 2);
   c->iw.ensure(nw + 1); c->iw_out.ensure(nw + 1); c->iw_hap0.ensure(nw + 1); c->ovf_list.ensure(nw + 1);
+  c->spq.ensure(nw + 1); c->spq_rp.ensure(nw + 1);  // a window is queued at most once
+  if (c->spill.cap == 0) c->spill.ensure(1 << 16);
   c->counters.ensure(mphk::CTR_COUNT); c->sums.ensure(3);
   {
     c->win_seg.ensure(nw + 1); c->tx_stop.ensure(b.txs.size() + 1);
@@ -399,7 +402,7 @@ void prepare(mph_ctx* c, const mph_batch* mb) {
   d.win_diff = c->win_diff.p; d.seg_list = c->seg_list.p; d.seg_list_n = c->seg_list_n.p; d.seg_list2_n = c->seg_list_n.p + b.segs.size() + 1; d.rr_seg0 = c->rr_seg0.p; d.ref = c->ref.p; d.stopmap = c->stopmap.p;
   d.call_S = reinterpret_cast<uint64_t*>(c->call_S.p); d.call_B = reinterpret_cast<uint64_t*>(c->call_B.p); d.call_flags = c->call_flags.p;
   d.win_out = c->win_out.p; d.hap0 = c->hap0.p; d.win_flag = c->win_flag.p; d.block_counts = c->block_counts.p;
-  d.ovf_list = c->ovf_list.p;
+  d.ovf_list = c->ovf_list.p; d.spq = c->spq.p; d.spq_rp = c->spq_rp.p;
   d.iw = c->iw.p; d.iw_out = c->iw_out.p; d.iw_hap0 = c->iw_hap0.p; d.counters = c->counters.p;
   d.sum_depth = c->sums.p; d.live_depth = c->sums.p + 1; d.seg_live = c->seg_live.p;
   d.window_len = b.window_len;
@@ -477,9 +480,10 @@ void set_ranges(mph_ctx* c, const Stage& s) {
 void run_kernels(mph_ctx* c) {
   if (!c->cur) throw std::runtime_error("no batch uploaded");
   mphk::DeviceBatch& d = c->d;
-  { const char* fw = getenv("MPH_FORCE_WIDE"); d.force_wide = (fw && *fw == '1') ? 1u : 0u; }
+  { const char* fw = getenv("MPH_FORCE_WIDE"); d.force_wide = (fw && (*fw == '1' || *fw == '2')) ? uint32_t(*fw - '0') : 0u; }
   if (c->hist_win.cap < c->hist.cap) c->hist_win.ensure(c->hist.cap);
   d.hist = c->hist.p; d.hapx = c->hapx.p; d.hist_win = c->hist_win.p; d.hist_cap = uint32_t(std::min<size_t>(c->hist.cap, 0xFFFFFFF0u));
+  d.spill = c->spill.p; d.spill_cap = uint32_t(std::min<size_t>(c->spill.cap, 0xFFFFFFF0u));
   d.seq = c->seq.p; d.seq_cap_bytes = uint32_t(std::min<size_t>(c->seq.cap, 0xFFFFFF00u));
   d.seq_dev = c->seq_dev.p; d.seq_dev_cap_bytes = uint32_t(std::min<size_t>(c->seq_dev.cap, 0xFFFFFF00u));
   d.recs = c->recs.p; d.rec_cap = uint32_t(std::min<size_t>(c->recs.cap, 0xFFFFFF00u));
@@ -619,7 +623,8 @@ void resize_pinned(mph_ctx* c, V& v, size_t n) {
 // an arena ran out during the last run_kernels (the counters say how much was asked for): grows it; true = run again
 bool grow_arenas(mph_ctx* c, const uint32_t* ctr) {
   const uint32_t err = ctr[mphk::CTR_ERR];
-  if (!(err & (MPH_E_HIST_OVERFLOW | MPH_E_SEQ_OVERFLOW | MPH_E_VLIST_OVERFLOW | MPH_E_REC_OVERFLOW))) return false;
+  if (!(err & (MPH_E_HIST_OVERFLOW | MPH_E_SEQ_OVERFLOW | MPH_E_VLIST_OVERFLOW | MPH_E_REC_OVERFLOW | MPH_E_SPILL_OVERFLOW))) return false;
+  if (err & MPH_E_SPILL_OVERFLOW) c->spill.ensure(size_t(ctr[mphk::CTR_SPILL]) * 2 + 1024);
   if (err & MPH_E_REC_OVERFLOW) {
     c->recs.ensure(std::max<size_t>(size_t(ctr[mphk::CTR_NREC]) * 2 + 1024, c->recs.cap));
     c->rec_seq.ensure(std::max<size_t>(size_t(ctr[mphk::CTR_RECSEQ]) * 2 + 4096, std::max(c->rec_seq.cap, c->recs.cap * 64)));
@@ -653,7 +658,8 @@ void fetch_stage(mph_ctx* c, const Stage& s, PhaseRaw& raw, uint64_t* n_iw_total
   if (raw.err & MPH_E_SEQ_SLOT) throw Unsupported("assembled haplotype longer than the sequence slot");
   if (raw.err & MPH_E_REF_RANGE) throw Fatal("slice index out of range: refseq");
   if (raw.err & MPH_E_VARS_PER_WINDOW) throw Unsupported("more than 32 variants in one window / 64 inside one read");
-  if (raw.err & MPH_E_KEYS_PER_WINDOW) throw Unsupported("more than 32 distinct haplotypes in one window");
+  if (raw.err & MPH_E_KEYS_PER_WINDOW) throw Unsupported(MPH_MSG_KEYS_PER_WINDOW);
+  if (raw.err & MPH_E_RECS_PER_LIST) throw Unsupported(MPH_MSG_RECS_PER_LIST);
   if (raw.err & MPH_E_REPLAY_PANIC) throw Fatal("bug: read starts right of variant");
   if (raw.err) throw std::logic_error("device error bits " + std::to_string(raw.err));
   const uint32_t n_iw = ctr[mphk::CTR_NIW], n_hist = ctr[mphk::CTR_HIST], n_seq = ctr[mphk::CTR_SEQ];

@@ -169,7 +169,7 @@ typedef struct {
 enum {
   MPH_E_HIST_OVERFLOW = 1,   // histogram arena exhausted -> host retries with a larger arena
   MPH_E_SEQ_OVERFLOW = 2,    // sequence arena exhausted  -> host retries with a larger arena
-  MPH_E_KEYS_PER_WINDOW = 4, // more distinct keys in one window than a warp table holds
+  MPH_E_KEYS_PER_WINDOW = 4, // more than MPH_BLOCK_KEYS distinct keys in one window
   MPH_E_REF_RANGE = 8,       // reference index out of the shipped slice (reference: slice panic)
   MPH_E_VARS_PER_WINDOW = 16, // > 64 variants in one window (reference: shift overflow)
   MPH_E_REPLAY_PANIC = 32,    // serial replay: the reference panics here (drain out of range, read right of a variant, inverted range)
@@ -178,5 +178,24 @@ enum {
   MPH_E_SLICE = 256,          // record kernels: a sequence slice the reference takes is out of range (reference: slice panic)
   MPH_E_INTERNAL = 512,       // record kernels: a haplotype that is written lacks its sequence or id
   MPH_E_SEQ_SLOT = 1024,      // assembled haplotype longer than the sequence slot / a record length field
-  MPH_E_REC_OVERFLOW = 2048   // record / merge arena exhausted -> host retries with larger arenas
+  MPH_E_REC_OVERFLOW = 2048,  // record / merge arena exhausted -> host retries with larger arenas
+  MPH_E_SPILL_OVERFLOW = 4096, // spill arena of the block histogram tier exhausted -> host retries with a larger arena
+  MPH_E_RECS_PER_LIST = 8192   // record kernels: more records from one window (4095) or one splice junction (MPH_RC_JUNCTION_RECS) than they index
 };
+
+// Third histogram tier: a window with more distinct keys than a warp table holds spills its counted observations
+// (MphHist entries, count = weight) to the spill arena and queues itself; k_window_hist_block (one CTA per queued window)
+// sorts and folds them in shared memory. MPH_BLOCK_KEYS distinct keys is what that buffer keeps: a window with more
+// raises MPH_E_KEYS_PER_WINDOW. The kernel, the CPU emulator and the error message share this bound.
+#define MPH_BLOCK_KEYS 4096
+#define MPH_XSTR_(x) #x
+#define MPH_XSTR(x) MPH_XSTR_(x)
+#define MPH_MSG_KEYS_PER_WINDOW "more than " MPH_XSTR(MPH_BLOCK_KEYS) " distinct haplotypes in one window"
+#define MPH_MSG_RECS_PER_LIST "more records from one window or one splice junction than a record list holds"
+
+// One queued window of the block tier, 16 B.
+typedef struct {
+  uint32_t code;    // (chunk << 5 | lane) of the window, as in hist_win
+  uint32_t off, n;  // its observations in the spill arena
+  uint32_t devrec;  // 1: the keys go to the back of the histogram arena (device-class transcript, somatic mode)
+} MphSpillWin;

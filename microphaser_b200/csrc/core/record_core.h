@@ -41,13 +41,17 @@ typedef struct {
   uint32_t var_ref;   // source A: first variant of its window
   uint32_t keep;      // source A: bit c <-> visited variant c passes the merge's position filter (all ones for a plain record)
   uint64_t profile;   // source A: 2 bits per visited variant, 0 absent, 1 germline, 2 somatic
-  uint8_t n_prof, n_win;  // source A: visited variants, variants in the window
-  uint8_t nvar, nsomatic, nsites, nsomsites;
-  uint8_t flags;      // MPH_RC_*
-  uint8_t rank;       // merged: position among the junction's records in output_map order
+  uint64_t n_prof : 7, n_win : 7;  // source A: visited variants, variants in the window (both <= 64)
+  uint64_t nvar : 8, nsomatic : 8, nsites : 8, nsomsites : 8;
+  uint64_t flags : 6;  // MPH_RC_*
+  uint64_t rank : 12;  // merged: position among the junction's records in output_map order (< MPH_RC_JUNCTION_RECS)
   uint8_t neo_len, mt_len, norm_len, wt_len;  // `mutant_sequence` column, mutant FASTA line, `normal_sequence` column, normal FASTA line
   uint32_t aux;       // merged: index of source B in the aux array
 } MphRec;
+#define MPH_RC_JUNCTION_RECS 4096  // records one splice junction may write (the width of `rank`); more raise MPH_E_RECS_PER_LIST
+#ifdef __cplusplus
+static_assert(sizeof(MphRec) == 64, "MphRec is 64 B");
+#endif
 
 typedef struct {  // source B of a merged record, 24 B
   uint64_t profile;
@@ -478,7 +482,7 @@ MPH_HD uint32_t mph_rc_merge_t(const MphRecCtx& c, const MphSegment& sp, const M
             Ops::load(win, ma, man, mb, ms, wa, wan, wb, ws, (uint32_t)wl);
             uint32_t slot = 0;
             for (; slot < n_out; ++slot) {
-              if (recs[slot].rank != (uint8_t)out_offset || recs[slot].aux != (uint32_t)out_offset) continue;  // rank / aux hold the key's offset until the final pass
+              if (recs[slot].aux != (uint32_t)out_offset) continue;  // aux holds the key's offset until the final pass
               if (Ops::equals_slot(win, seq + seq_base + (size_t)slot * MPH_RC_SEQ_SLOT, (uint32_t)wl)) break;
             }
             double old_freq = 0.0;
@@ -513,7 +517,7 @@ MPH_HD uint32_t mph_rc_merge_t(const MphRecCtx& c, const MphSegment& sp, const M
             r.seq_off = seq_base + slot * MPH_RC_SEQ_SLOT;
             r.var_ref = self.var_ref; r.keep = ka; r.profile = self.profile; r.n_prof = self.n_prof; r.n_win = self.n_win;
             r.flags = (uint8_t)(MPH_RC_MERGED | MPH_RC_HAS_MT | MPH_RC_HAS_WT | (fwd ? 0 : MPH_RC_REVERSE));
-            r.rank = (uint8_t)out_offset;
+            r.rank = 0;
             r.neo_len = r.mt_len = r.norm_len = r.wt_len = (uint8_t)wl;
             r.aux = (uint32_t)out_offset;
             if (Ops::leader()) recs[slot] = r;
@@ -530,6 +534,7 @@ MPH_HD uint32_t mph_rc_merge_t(const MphRecCtx& c, const MphSegment& sp, const M
   }
   if (recs) {
     // ranks in output_map order: (out_offset, mt bytes, wt bytes) (:1518-1521); then aux takes its final meaning
+    if (n_out > MPH_RC_JUNCTION_RECS) { *err |= MPH_E_RECS_PER_LIST; return 0; }
     for (uint32_t x = 0; x < n_out; ++x) {
       uint32_t rank = 0;
       const uint8_t* sx = seq + seq_base + (size_t)x * MPH_RC_SEQ_SLOT;
@@ -541,7 +546,7 @@ MPH_HD uint32_t mph_rc_merge_t(const MphRecCtx& c, const MphSegment& sp, const M
         else less = Ops::slot_less(sy, sx, (uint32_t)(2 * wl));
         if (less) ++rank;
       }
-      if (Ops::leader()) recs[x].rank = (uint8_t)rank;
+      if (Ops::leader()) recs[x].rank = rank;
     }
     Ops::sync();
     if (Ops::leader())
@@ -826,7 +831,8 @@ MPH_HD uint32_t mph_nrc_merge_t(const MphRecCtx& c, const MphNrmCtx& n, const Mp
     }
   }
   if (recs) {
-    // ranks in output_map order: (splice_offset, out_seq) (:1216-1222)
+    // ranks in output_map order: (splice_offset, out_seq) (:1216-1222); then aux takes its final meaning
+    if (n_out > MPH_RC_JUNCTION_RECS) { *err |= MPH_E_RECS_PER_LIST; return 0; }
     for (uint32_t x = 0; x < n_out; ++x) {
       uint32_t rank = 0;
       const uint8_t* sx = seq + seq_base + (size_t)x * MPH_RC_SEQ_SLOT;
@@ -838,7 +844,7 @@ MPH_HD uint32_t mph_nrc_merge_t(const MphRecCtx& c, const MphNrmCtx& n, const Mp
         else less = Ops::slot_less(sy, sx, (uint32_t)wl);
         if (less) ++rank;
       }
-      if (Ops::leader()) recs[x].rank = (uint8_t)rank;
+      if (Ops::leader()) recs[x].rank = rank;
     }
     Ops::sync();
     if (Ops::leader())

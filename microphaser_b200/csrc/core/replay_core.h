@@ -33,7 +33,7 @@ typedef struct {
   uint32_t pad;
 } MphReplayTx;
 
-typedef struct {
+typedef struct MphReplayCtx {
   // inputs (same arrays as the closed-form kernels)
   const uint32_t* read_start; const uint32_t* read_end; const uint8_t* read_flags;
   const uint32_t* read_vlo; const uint8_t* read_nv; const uint32_t* read_vr;  // per read, expanded by K1 from the compact side table (read_vr = its entry)
@@ -54,6 +54,7 @@ typedef struct {
   uint8_t* o_inmat;  // per gene read (obs_off + read - read_lo): the read is an observation right now
   // outputs
   MphWinOut* win_out; MphHist* hist; uint32_t* hist_win; uint32_t hist_cap;
+  uint32_t key_cap = MPH_RP_KEYS;  // keys of the window table before a window is sorted in the arena instead (0 under MPH_FORCE_WIDE=2)
   MphHap* hap0; uint8_t* win_flag;
   uint32_t* win_voff;  // per window: offset of its column list in vlist (entry 0 = count), 0xFFFFFFFF = the window's own variants
   uint32_t* vlist; uint32_t vlist_cap;
@@ -141,6 +142,33 @@ MPH_HD uint32_t mph_rp_partner(const MphReplayCtx& c, uint32_t r) {
   return (lo < c.n_pairs && c.pairs[2 * lo] == r) ? c.pairs[2 * lo + 1] : 0xFFFFFFFFu;
 }
 
+// BTreeMap order of the keys (:383,434): haplotype, frame.0, frame.1 != 0
+MPH_HD bool mph_rp_hist_less(const MphHist& a, const MphHist& b) {
+  if (a.hap != b.hap) return a.hap < b.hap;
+  const uint32_t fa = a.frame & 0x7FFFFFFFu, fb = b.frame & 0x7FFFFFFFu;
+  if (fa != fb) return fa < fb;
+  return (a.frame >> 31) < (b.frame >> 31);
+}
+
+// in-place heapsort of h[0, n) in that order (serial, no scratch)
+MPH_HD void mph_rp_heapsort(MphHist* h, uint32_t n) {
+  auto sift = [&](uint32_t root, uint32_t end) {
+    for (;;) {
+      uint32_t child = 2 * root + 1;
+      if (child >= end) return;
+      if (child + 1 < end && mph_rp_hist_less(h[child], h[child + 1])) ++child;
+      if (!mph_rp_hist_less(h[root], h[child])) return;
+      const MphHist tmp = h[root]; h[root] = h[child]; h[child] = tmp;
+      root = child;
+    }
+  };
+  for (uint32_t r = n / 2; r-- > 0;) sift(r, n);
+  for (uint32_t end = n; end > 1; --end) {
+    const MphHist tmp = h[0]; h[0] = h[end - 1]; h[end - 1] = tmp;
+    sift(0, end - 1);
+  }
+}
+
 // histogram + outputs of one enumerated window (the part of print_haplotypes :383-411 that reads the matrix)
 MPH_HD void mph_rp_emit(const MphReplayCtx& c, const MphReplayTx& t, const MphSegment& sg, uint32_t si, uint32_t i, uint32_t k, const MphGeom& g,
                         uint32_t n_obs, const uint32_t* dq, uint32_t ncols, uint32_t* err) {
@@ -149,6 +177,7 @@ MPH_HD void mph_rp_emit(const MphReplayCtx& c, const MphReplayTx& t, const MphSe
   uint32_t n_keys = 0, c0 = 0;
   const bool normal = c.mode == 1;
   uint32_t depth = normal ? 0u : n_obs;
+  bool spill = false;    // more keys than the table holds
   for (uint32_t o = 0; o < n_obs; ++o) {
     if (c.o_flags[t.obs_off + o] & 1) continue;
     const uint64_t hap = c.o_hap[t.obs_off + o];
@@ -156,24 +185,22 @@ MPH_HD void mph_rp_emit(const MphReplayCtx& c, const MphReplayTx& t, const MphSe
     const uint32_t fr = normal ? 0u : c.o_frame[t.obs_off + o];
     if (normal) depth += wgt;
     if (hap == 0 && fr == 0) { c0 += wgt; continue; }
+    if (spill) continue;
     uint32_t x = 0;
     for (; x < n_keys; ++x)
       if (table[x].hap == hap && table[x].frame == fr) break;
     if (x == n_keys) {
-      if (n_keys == MPH_RP_KEYS) { *err |= MPH_E_KEYS_PER_WINDOW; continue; }
+      if (n_keys == c.key_cap) { spill = true; continue; }
       table[x].hap = hap; table[x].frame = fr; table[x].count = 0;
       ++n_keys;
     }
     table[x].count += wgt;
   }
+  const uint32_t code = ((c.seg_chunk0[si] + (i >> 5)) << 5) | (i & 31u);
   for (uint32_t a = 1; a < n_keys; ++a) {  // BTreeMap order (:383,434): haplotype, frame.0, frame.1 != 0
     const MphHist key = table[a];
     uint32_t b = a;
-    while (b > 0) {
-      const MphHist& p = table[b - 1];
-      const uint32_t fa = key.frame & 0x7FFFFFFFu, fb = p.frame & 0x7FFFFFFFu;
-      const bool less = key.hap != p.hap ? key.hap < p.hap : (fa != fb ? fa < fb : (key.frame >> 31) < (p.frame >> 31));
-      if (!less) break;
+    while (b > 0 && mph_rp_hist_less(key, table[b - 1])) {
       table[b] = table[b - 1];
       --b;
     }
@@ -184,11 +211,52 @@ MPH_HD void mph_rp_emit(const MphReplayCtx& c, const MphReplayTx& t, const MphSe
   wo.c0 = c0;
   wo.n_extra = n_keys;
   wo.extra_off = 0;
-  if (n_keys) {
+  if (spill) {
+    // more keys than the table holds (the block tier's serial statement): the window's distinct keys, counted without
+    // scratch (a key is listed at its first observation, with the weights of all its observations), are sorted in the key arena
+    auto counted = [&](uint32_t o) {
+      return !(c.o_flags[t.obs_off + o] & 1) && (c.o_hap[t.obs_off + o] != 0 || (!normal && c.o_frame[t.obs_off + o] != 0));
+    };
+    auto same = [&](uint32_t o, uint32_t q) {
+      return c.o_hap[t.obs_off + o] == c.o_hap[t.obs_off + q] && (normal || c.o_frame[t.obs_off + o] == c.o_frame[t.obs_off + q]);
+    };
+    auto first = [&](uint32_t o) {
+      for (uint32_t q = 0; q < o; ++q)
+        if (counted(q) && same(o, q)) return false;
+      return true;
+    };
+    uint32_t n_fold = 0;
+    for (uint32_t o = 0; o < n_obs; ++o) n_fold += (counted(o) && first(o)) ? 1u : 0u;
+    wo.n_extra = 0;
+    if (n_fold > MPH_BLOCK_KEYS) {
+      *err |= MPH_E_KEYS_PER_WINDOW;
+    } else {
+      const uint32_t off = MPH_RP_ADD(&c.counters[MPH_RP_CTR_HIST], n_fold);
+      if (off + n_fold <= c.hist_cap) {
+        MphHist* h = c.hist + off;
+        uint32_t y = 0;
+        for (uint32_t o = 0; o < n_obs; ++o) {
+          if (!counted(o) || !first(o)) continue;
+          MphHist e;
+          e.hap = c.o_hap[t.obs_off + o];
+          e.frame = normal ? 0u : c.o_frame[t.obs_off + o];
+          e.count = 0;
+          for (uint32_t q = o; q < n_obs; ++q)
+            if (counted(q) && same(o, q)) e.count += normal ? c.o_frame[t.obs_off + q] : 1u;
+          c.hist_win[off + y] = code;
+          h[y++] = e;
+        }
+        mph_rp_heapsort(h, n_fold);
+        wo.n_extra = n_fold;
+        wo.extra_off = off;
+      } else {
+        *err |= MPH_E_HIST_OVERFLOW;
+      }
+    }
+  } else if (n_keys) {
     const uint32_t off = MPH_RP_ADD(&c.counters[MPH_RP_CTR_HIST], n_keys);
     if (off + n_keys <= c.hist_cap) {
       wo.extra_off = off;
-      const uint32_t code = ((c.seg_chunk0[si] + (i >> 5)) << 5) | (i & 31u);
       for (uint32_t a = 0; a < n_keys; ++a) {
         c.hist[off + a] = table[a];
         c.hist_win[off + a] = code;

@@ -94,6 +94,8 @@ inline int run_somatic(int argc, char** argv, const PhaseFn& phase) {
   if (raw.err & MPH_E_VARS_PER_WINDOW) throw Unsupported("more than 32 variants in one window / 64 in one read");
   if (raw.err & MPH_E_SLICE) throw Fatal("slice index out of range");
   if (raw.err & MPH_E_SEQ_SLOT) throw Unsupported("assembled haplotype longer than the sequence slot");
+  if (raw.err & MPH_E_KEYS_PER_WINDOW) throw Unsupported(MPH_MSG_KEYS_PER_WINDOW);
+  if (raw.err & MPH_E_RECS_PER_LIST) throw Unsupported(MPH_MSG_RECS_PER_LIST);
   if (raw.err) throw std::runtime_error("device error bits " + std::to_string(raw.err));
   Residue res(b, raw);
   std::vector<OutRecord> host_recs;
@@ -132,6 +134,8 @@ inline int run_normal(int argc, char** argv, const PhaseFn& phase) {
   PhaseRaw raw = phase(b);
   if (raw.err & MPH_E_REF_RANGE) throw Fatal("index out of bounds: refseq");
   if (raw.err & MPH_E_VARS_PER_WINDOW) throw Unsupported("more than 32 variants in one window / 64 in one read");
+  if (raw.err & MPH_E_KEYS_PER_WINDOW) throw Unsupported(MPH_MSG_KEYS_PER_WINDOW);
+  if (raw.err & MPH_E_RECS_PER_LIST) throw Unsupported(MPH_MSG_RECS_PER_LIST);
   if (raw.err) throw std::runtime_error("device error bits " + std::to_string(raw.err));
   if (raw.err & MPH_E_SLICE) throw Fatal("slice index out of range");
   if (raw.err & MPH_E_SEQ_SLOT) throw Unsupported("assembled haplotype longer than the sequence slot");

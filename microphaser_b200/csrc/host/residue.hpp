@@ -363,7 +363,8 @@ class Residue {
     // histogram for this frame (:383-411) from the fine keys (hap, obs.frame.0, obs.frame.1 != 0)
     // device keys arrive sorted by (hap, obs.frame.0, obs.frame.1 != 0); projecting them onto this frame's
     // (hap, frame) key keeps the order, equal keys become adjacent -> a small sorted vector, no tree
-    Key keybuf[40];
+    std::vector<Key>& keybuf = key_scratch_;  // reused across windows; a window may have any number of keys
+    keybuf.clear();
     size_t n_keys = 0;
     uint64_t frame_depth = 0;
     auto add = [&](uint64_t hap, uint32_t fr, uint64_t count, const MphHap* info) {
@@ -376,8 +377,8 @@ class Residue {
         if (keybuf[q].hap == hap && keybuf[q].frame == kf) { keybuf[q].count += count; return; }
         if (keybuf[q].hap != hap) break;
       }
-      if (n_keys == 40) throw Unsupported("more than 40 haplotype keys in one window");
-      keybuf[n_keys++] = Key{hap, kf, count, info};
+      keybuf.push_back(Key{hap, kf, count, info});
+      ++n_keys;
     };
     if (wo.c0 > 0) add(0, 0, wo.c0, &h0);
     for (uint32_t x = 0; x < wo.n_extra; ++x) {
@@ -393,7 +394,7 @@ class Residue {
       keybuf[z] = kq;
     }
     const bool has_frameshift = frame > 0;
-    if (n_keys == 0) keybuf[n_keys++] = Key{0, 0, 0, &h0};
+    if (n_keys == 0) { keybuf.push_back(Key{0, 0, 0, &h0}); ++n_keys; }
     if (trace_) {  // same line format as the oracle's MPH_ORACLE_TRACE
       fprintf(trace_, "W\t%s\t%llu\t%llu\t%llu\t%u\t%llu\t%u", tm.id.c_str(), (unsigned long long)g.s, (unsigned long long)g.e,
               (unsigned long long)frame_in, wo.depth, (unsigned long long)frame_depth, nv);
@@ -950,6 +951,7 @@ class Residue {
   InfoRecord unused_rec_;  // what `rec` names in print() for a haplotype that needs no record; never written
   size_t iw_lo_ = 0, iw_hi_ = 0, iw_hint_ = 0;  // this segment's slice of raw_.iw and the last lookup (find_iw)
   std::vector<uint32_t> ks_scratch_;
+  std::vector<Key> key_scratch_;  // print(): the window's keys projected onto one frame
 };
 
 }  // namespace mph

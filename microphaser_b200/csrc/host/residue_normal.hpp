@@ -136,30 +136,28 @@ class ResidueNormal {
     const uint64_t window_len = sg.ewl;
     const uint32_t wd = raw_.win_depth[widx - raw_.win_base];
     const uint32_t depth = wd & 0x7FFFFFFFu;
-    struct Key { uint64_t hap; uint64_t count; const MphHap* info; };
-    Key keybuf[64];
-    size_t n_keys = 0;
+    std::vector<Key>& keybuf = key_scratch_;  // reused across windows; a window may have any number of keys
+    keybuf.clear();
     MphHap plain;
     if (nv == 0) {
       memset(&plain, 0, sizeof plain);
       plain.flags = (wd >> 31) ? MPH_NF_STOP : 0;
       plain.seq_len = uint16_t(g.e - g.s);
-      keybuf[n_keys++] = Key{0, depth, &plain};
+      keybuf.push_back(Key{0, depth, &plain});
     } else {
       if (iwi == SIZE_MAX) iwi = find_iw(widx);
       if (iwi == SIZE_MAX) throw std::logic_error("internal: window summary missing");
       const MphWinOut& wo = raw_.iw_out[iwi];
-      if (wo.c0 > 0) keybuf[n_keys++] = Key{0, wo.c0, &raw_.iw_hap0[iwi]};
-      if (wo.n_extra > 63) throw Unsupported("more than 63 haplotypes in one window");
+      if (wo.c0 > 0) keybuf.push_back(Key{0, wo.c0, &raw_.iw_hap0[iwi]});
       for (uint32_t x = 0; x < wo.n_extra; ++x) {
         const MphHist& e = raw_.hist[wo.extra_off + x];
-        keybuf[n_keys++] = Key{e.hap, e.count, &raw_.hapx[wo.extra_off + x]};
+        keybuf.push_back(Key{e.hap, e.count, &raw_.hapx[wo.extra_off + x]});
       }
-      if (n_keys == 0) keybuf[n_keys++] = Key{0, 0, &raw_.iw_hap0[iwi]};
+      if (keybuf.empty()) keybuf.push_back(Key{0, 0, &raw_.iw_hap0[iwi]});
     }
     std::vector<HapSeq> res;
     *n_res = 0;
-    for (size_t q = 0; q < n_keys; ++q) {
+    for (size_t q = 0; q < keybuf.size(); ++q) {
       const Key& key = keybuf[q];
       const MphHap& h = *key.info;
       if (h.flags & MPH_NF_REFRANGE) throw Fatal("index out of bounds: refseq");  // the reference panics when it reaches this walk
@@ -393,8 +391,10 @@ class ResidueNormal {
     }
   }
 
+  struct Key { uint64_t hap; uint64_t count; const MphHap* info; };
   const Batch& b_;
   const PhaseRaw& raw_;
+  std::vector<Key> key_scratch_;  // print(): the window's keys
 };
 
 }  // namespace mph

@@ -53,6 +53,8 @@ __device__ __forceinline__ uint32_t normal_rev_kc(const MphSegment& sg, uint32_t
   return kc;
 }
 
+// one warp per window whose keys overflow a lane table; a window with more keys than the warp table holds walks its reads a
+// second time and hands its haplotypes to k_window_hist_block (as in window_hist_warp of phase_kernels.cu)
 __device__ void window_hist_warp_normal(const DeviceBatch& d, const MphSegment& sg, uint32_t ch_seg, uint32_t i, uint32_t code, MphHist* table, int lane) {
   const bool rev = (sg.flags & MPH_SF_REVERSE) != 0;
   const uint32_t k = sg.k_first + i * sg.k_stride;
@@ -62,22 +64,27 @@ __device__ void window_hist_warp_normal(const DeviceBatch& d, const MphSegment& 
   const uint32_t vb = mph_var_lb(d.vars, va, sg.var_hi, g.e);
   uint32_t rlo, rhi;
   mph_candidate_range(sg, d.read_start, g, &rlo, &rhi);
-  uint32_t depth = 0, c0 = 0, n_keys = 0;
-  for (uint32_t base = rlo; base < rhi; base += 32) {
-    const uint32_t r = base + lane;
-    uint32_t copies = 0, kp_last = k, vlo = 0;
-    uint64_t S = 0;
-    if (r < rhi) {
-      const uint32_t st = d.read_start[r], en = d.read_end[r];
-      if (!rev) {
-        const uint32_t kp = mph_nrm_fwd_entry(sg, k, g, st, en);
-        if (kp != NONE) { copies = 1; kp_last = kp; }
-      } else {
-        uint32_t kc;
-        copies = mph_nrm_rev_copies(sg, k, g, st, en, &kc);
-      }
-      if (copies && (d.call_flags[r] & 1u)) { S = d.call_S[r]; vlo = d.read_vlo[r]; }  // S is only written for reads with a call
+  // the copies of read r in the matrix; S != 0: they need their haplotypes
+  auto observe = [&](uint32_t r, uint32_t* copies, uint32_t* kp_last, uint32_t* vlo, uint64_t* S) {
+    *copies = 0; *kp_last = k; *vlo = 0; *S = 0;
+    if (r >= rhi) return;
+    const uint32_t st = d.read_start[r], en = d.read_end[r];
+    if (!rev) {
+      const uint32_t kp = mph_nrm_fwd_entry(sg, k, g, st, en);
+      if (kp != NONE) { *copies = 1; *kp_last = kp; }
+    } else {
+      uint32_t kc;
+      *copies = mph_nrm_rev_copies(sg, k, g, st, en, &kc);
     }
+    if (*copies && (d.call_flags[r] & 1u)) { *S = d.call_S[r]; *vlo = d.read_vlo[r]; }  // S is only written for reads with a call
+  };
+  const uint32_t key_cap = d.force_wide == 2 ? 0u : (uint32_t)K2_TABLE;
+  uint32_t depth = 0, c0 = 0, n_keys = 0, n_spill = 0;
+  bool spill = false;  // lane 0: a key did not fit the table
+  for (uint32_t base = rlo; base < rhi; base += 32) {
+    uint32_t copies, kp_last, vlo;
+    uint64_t S;
+    observe(base + lane, &copies, &kp_last, &vlo, &S);
     uint32_t cs = copies;
     for (int o = 16; o; o >>= 1) cs += __shfl_xor_sync(FULL, cs, o);
     depth += cs;
@@ -93,30 +100,67 @@ __device__ void window_hist_warp_normal(const DeviceBatch& d, const MphSegment& 
       if (have) hap = mph_nrm_hap(sg, d.vars, rev ? k - c : kp_last, k, va, vb, vlo, S);
       c0 += __popc(__ballot_sync(FULL, have && hap == 0));
       unsigned pending = __ballot_sync(FULL, have && hap != 0);
+      n_spill += __popc(pending);
+      if (__shfl_sync(FULL, (int)spill, 0)) continue;
       while (pending) {
         const int leader = __ffs(pending) - 1;
         const uint64_t lh = __shfl_sync(FULL, hap, leader);
         const unsigned same = __ballot_sync(FULL, have && hap == lh);
-        if (lane == 0) {
+        if (lane == 0 && !spill) {
           uint32_t t = 0;
           for (; t < n_keys; ++t)
             if (table[t].hap == lh) break;
           if (t == n_keys) {
-            if (n_keys < K2_TABLE) {
+            if (n_keys < key_cap) {
               table[t].hap = lh;
               table[t].frame = 0;
               table[t].count = 0;
               ++n_keys;
             } else {
-              raise(d, MPH_E_KEYS_PER_WINDOW);
-              t = K2_TABLE - 1;
+              spill = true;
             }
           }
-          table[t].count += __popc(same);
+          if (!spill) table[t].count += __popc(same);
         }
         pending &= ~same;
       }
     }
+  }
+  if (__shfl_sync(FULL, (int)spill, 0)) {
+    uint32_t off = 0;
+    if (lane == 0) off = atomicAdd(&d.counters[CTR_SPILL], n_spill);
+    off = __shfl_sync(FULL, off, 0);
+    if ((uint64_t)off + n_spill <= d.spill_cap) {
+      uint32_t y = off;
+      for (uint32_t base = rlo; base < rhi; base += 32) {
+        uint32_t copies, kp_last, vlo;
+        uint64_t S;
+        observe(base + lane, &copies, &kp_last, &vlo, &S);
+        uint32_t todo = (S != 0) ? copies : 0, maxc = todo;
+        for (int o = 16; o; o >>= 1) maxc = max(maxc, __shfl_xor_sync(FULL, maxc, o));
+        for (uint32_t c = 0; c < maxc; ++c) {
+          const bool have = c < todo;
+          uint64_t hap = 0;
+          if (have) hap = mph_nrm_hap(sg, d.vars, rev ? k - c : kp_last, k, va, vb, vlo, S);
+          const bool emit = have && hap != 0;
+          const unsigned bal = __ballot_sync(FULL, emit);
+          if (emit) {
+            MphHist e;
+            e.hap = hap; e.count = 1; e.frame = 0;
+            d.spill[y + __popc(bal & ((1u << lane) - 1u))] = e;
+          }
+          y += __popc(bal);
+        }
+      }
+      if (lane == 0) {
+        MphSpillWin q;
+        q.code = code; q.off = off; q.n = n_spill; q.devrec = 0;  // normal mode: every key sits at the front of the arena
+        d.spq[atomicAdd(&d.counters[CTR_SPQ], 1u)] = q;
+      }
+    } else if (lane == 0) {
+      raise(d, MPH_E_SPILL_OVERFLOW);
+    }
+    n_keys = 0;  // k_window_hist_block writes the keys and sets n_extra / extra_off
   }
   if (lane == 0) {
     for (uint32_t a = 1; a < n_keys; ++a) {  // ascending haplotype value (VecMap iteration order :383)
@@ -421,6 +465,7 @@ void launch_window_hist_normal(const DeviceBatch& d, cudaStream_t st) {
   MPH_LAUNCH(k_window_hist_normal, ((nc + K2_WARPS - 1) / K2_WARPS, K2_WARPS * 32, 0, st), d);
   // windows with more distinct haplotypes than a lane table holds (rare): one warp per window
   MPH_LAUNCH(k_window_hist_wide_normal, (148 * 8, K2_WARPS * 32, 0, st), d);
+  launch_window_hist_block(d, st, SPQ_K2);  // ... and those with more keys than a warp table holds: one CTA per window
 }
 void launch_assemble_normal(const DeviceBatch& d, cudaStream_t st) {
   MPH_LAUNCH(k_assemble_normal, (148 * 8, 128, 0, st), d);  // grid-stride over the key arena (its size lives on the device)

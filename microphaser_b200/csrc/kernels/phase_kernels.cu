@@ -9,7 +9,8 @@
 //                      grid) and a list of the reads that carry allele calls; thread = window prefix-sums it into
 //                      depth and evaluates the closed form of the ObservationMatrix (:157-343) for the listed reads
 //                      only; haplotype keys go to per-window shared-memory tables (:383-411). k_window_hist_wide
-//                      redoes windows whose keys overflow a table, one warp per window.
+//                      redoes windows whose keys overflow a table, one warp per window, and k_window_hist_block
+//                      (block_kernels.cu) the few whose keys overflow that warp's table, one CTA per window.
 //   K3 k_assemble      thread per extra haplotype key: sequence walk (:458-603), stop codon test (:42-76,
 //                      :694-697) and the SHA-1 record id (:667-675) while the bytes are in registers / L1.
 //   K4 k_flag_count / k_block_scan / k_scatter   stable compaction of the interesting windows so the
@@ -160,7 +161,8 @@ __device__ __forceinline__ MphPair eval_flagged(const DeviceBatch& d, const MphS
 }
 
 // Wide variant: one warp per window, lanes over the candidate reads, keys in a 32-entry table.
-// Used only for windows whose key count overflows the per-lane table of k_window_hist.
+// Used only for windows whose key count overflows the per-lane table of k_window_hist. A window with more keys than the
+// table holds walks its reads a second time and hands its counted observations to k_window_hist_block (spill_window).
 __device__ void window_hist_warp(const DeviceBatch& d, const MphSegment& sg, uint32_t ch_seg, uint32_t i, uint32_t code, MphHist* table, int lane) {
   const bool rev = (sg.flags & MPH_SF_REVERSE) != 0;
   const uint32_t k = sg.k_first + i * sg.k_stride;
@@ -170,52 +172,88 @@ __device__ void window_hist_warp(const DeviceBatch& d, const MphSegment& sg, uin
   const uint32_t vb = mph_var_lb(d.vars, va, sg.var_hi, g.e);
   uint32_t rlo, rhi;
   mph_candidate_range(sg, d.read_start, g, &rlo, &rhi);
-  uint32_t depth = 0, c0 = 0, n_keys = 0;
+  // the observation of read r (member / counted = member and not bad_qual) with its key
+  auto observe = [&](uint32_t r, bool* member, bool* counted, uint64_t* hap, uint32_t* frame) {
+    *member = false; *counted = false; *hap = 0; *frame = 0;
+    if (r >= rhi) return;
+    const uint32_t st = d.read_start[r], en = d.read_end[r];
+    if (en < g.e) return;
+    const uint32_t cf = d.call_flags[r] | ((d.read_flags[r] & MPH_RF_PARTNER) ? 2u : 0u);
+    const uint64_t S = (cf & 1u) ? d.call_S[r] : 0, B = (cf & 1u) ? d.call_B[r] : 0;  // S / B are only written for reads with a call
+    const MphPair p = eval_flagged(d, sg, rev, k, g, va, vb, r, st, en, cf, d.read_vlo[r], S, B);
+    *member = p.member != 0;
+    *counted = *member && !p.bad;
+    *hap = p.hap;
+    *frame = p.frame;
+  };
+  const uint32_t key_cap = d.force_wide == 2 ? 0u : (uint32_t)K2_TABLE;
+  uint32_t depth = 0, c0 = 0, n_keys = 0, n_spill = 0;
+  bool spill = false;  // lane 0: a key did not fit the table
   for (uint32_t base = rlo; base < rhi; base += 32) {
-    const uint32_t r = base + lane;
-    bool member = false, counted = false;
-    uint64_t hap = 0;
-    uint32_t frame = 0;
-    if (r < rhi) {
-      const uint32_t st = d.read_start[r], en = d.read_end[r];
-      if (en >= g.e) {
-        const uint32_t cf = d.call_flags[r] | ((d.read_flags[r] & MPH_RF_PARTNER) ? 2u : 0u);
-        const uint64_t S = (cf & 1u) ? d.call_S[r] : 0, B = (cf & 1u) ? d.call_B[r] : 0;  // S / B are only written for reads with a call
-        const MphPair p = eval_flagged(d, sg, rev, k, g, va, vb, r, st, en, cf, d.read_vlo[r], S, B);
-        member = p.member != 0;
-        counted = member && !p.bad;
-        hap = p.hap;
-        frame = p.frame;
-      }
-    }
+    bool member, counted;
+    uint64_t hap;
+    uint32_t frame;
+    observe(base + lane, &member, &counted, &hap, &frame);
     depth += __popc(__ballot_sync(FULL, member));
     const bool zero_key = counted && hap == 0 && frame == 0;
     c0 += __popc(__ballot_sync(FULL, zero_key));
     unsigned pending = __ballot_sync(FULL, counted && !zero_key);
+    n_spill += __popc(pending);
+    if (__shfl_sync(FULL, (int)spill, 0)) continue;
     while (pending) {
       const int leader = __ffs(pending) - 1;
       const uint64_t lh = __shfl_sync(FULL, hap, leader);
       const uint32_t lf = __shfl_sync(FULL, frame, leader);
       const unsigned same = __ballot_sync(FULL, counted && !zero_key && hap == lh && frame == lf);
-      if (lane == 0) {
+      if (lane == 0 && !spill) {
         uint32_t t = 0;
         for (; t < n_keys; ++t)
           if (table[t].hap == lh && table[t].frame == lf) break;
         if (t == n_keys) {
-          if (n_keys < K2_TABLE) {
+          if (n_keys < key_cap) {
             table[t].hap = lh;
             table[t].frame = lf;
             table[t].count = 0;
             ++n_keys;
           } else {
-            raise(d, MPH_E_KEYS_PER_WINDOW);
-            t = K2_TABLE - 1;
+            spill = true;
           }
         }
-        table[t].count += __popc(same);
+        if (!spill) table[t].count += __popc(same);
       }
       pending &= ~same;
     }
+  }
+  if (__shfl_sync(FULL, (int)spill, 0)) {
+    // second walk: the counted observations outside the (0, 0) key, in read order, to the spill arena
+    uint32_t off = 0;
+    if (lane == 0) off = atomicAdd(&d.counters[CTR_SPILL], n_spill);
+    off = __shfl_sync(FULL, off, 0);
+    if ((uint64_t)off + n_spill <= d.spill_cap) {
+      uint32_t y = off;
+      for (uint32_t base = rlo; base < rhi; base += 32) {
+        bool member, counted;
+        uint64_t hap;
+        uint32_t frame;
+        observe(base + lane, &member, &counted, &hap, &frame);
+        const bool emit = counted && !(hap == 0 && frame == 0);
+        const unsigned bal = __ballot_sync(FULL, emit);
+        if (emit) {
+          MphHist e;
+          e.hap = hap; e.count = 1; e.frame = frame;
+          d.spill[y + __popc(bal & ((1u << lane) - 1u))] = e;
+        }
+        y += __popc(bal);
+      }
+      if (lane == 0) {
+        MphSpillWin q;
+        q.code = code; q.off = off; q.n = n_spill; q.devrec = (sg.flags & MPH_SF_DEVREC) ? 1u : 0u;
+        d.spq[atomicAdd(&d.counters[CTR_SPQ], 1u)] = q;
+      }
+    } else if (lane == 0) {
+      raise(d, MPH_E_SPILL_OVERFLOW);
+    }
+    n_keys = 0;  // k_window_hist_block writes the keys and sets n_extra / extra_off
   }
   if (lane == 0) {
     for (uint32_t a = 1; a < n_keys; ++a) {  // keys in the reference's BTreeMap order (:383,434)
@@ -782,6 +820,7 @@ void launch_window_hist(const DeviceBatch& d, cudaStream_t st) {
   else MPH_LAUNCH(k_window_hist<8>, ((nc + K2B_WARPS - 1) / K2B_WARPS, K2B_WARPS * 32, 0, st), d);
   // windows with more distinct haplotypes than a lane table holds (rare): one warp per window
   MPH_LAUNCH(k_window_hist_wide, (148 * 8, K2_WARPS * 32, 0, st), d);
+  launch_window_hist_block(d, st, SPQ_K2);  // ... and those with more keys than a warp table holds: one CTA per window
 }
 void launch_assemble(const DeviceBatch& d, cudaStream_t st, int part) {
   if (d.c1 > d.c0 && d.mode == 1) launch_assemble_normal(d, st);

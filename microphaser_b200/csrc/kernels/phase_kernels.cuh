@@ -23,7 +23,9 @@ struct DeviceBatch {
   uint32_t w0 = 0, w1 = 0;    // windows (K4)
   uint32_t rp0 = 0, rp1 = 0;  // replay units
   uint32_t mode = 0;        // 0 somatic, 1 normal (reference src/normal_microphasing.rs)
-  uint32_t force_wide = 0;  // test hook (MPH_FORCE_WIDE=1): send every window with extra keys through k_window_hist_wide
+  // test hook MPH_FORCE_WIDE: 1 sends every window with extra keys through k_window_hist_wide; 2 also makes the wide kernels
+  // and the replay spill such a window at its first extra key, so that every one of them goes through k_window_hist_block
+  uint32_t force_wide = 0;
   const uint32_t* read_start = nullptr;  // rebuilt on the device by K0 from the 2-byte bus encoding below
   const uint32_t* read_end = nullptr;
   const uint8_t* read_flags = nullptr;
@@ -89,6 +91,13 @@ struct DeviceBatch {
   uint32_t hist_cap = 0;          // keys of host-class windows fill the arena from the front (CTR_HIST, downloaded), those of
                                   // device-class transcripts from the back (CTR_HISTD, read by K3 and the record kernels only)
   uint32_t* ovf_list = nullptr;  // (chunk << 5 | lane) of windows whose keys overflow a lane table; chunk count must be < 2^27
+  // block tier (layout.h MPH_BLOCK_KEYS): windows whose keys overflow a warp table. The wide kernels and the replay append their
+  // counted observations to `spill` (counters[CTR_SPILL] entries) and queue them: K2's in spq (counters[CTR_SPQ]), the replay's
+  // in spq_rp (counters[CTR_SPQR]); a window is queued at most once, so a queue of n_windows entries cannot overflow
+  MphHist* spill = nullptr;
+  uint32_t spill_cap = 0;
+  MphSpillWin* spq = nullptr;
+  MphSpillWin* spq_rp = nullptr;
   // K3 output
   MphHap* hap0 = nullptr;
   MphHap* hapx = nullptr;  // parallel to hist
@@ -142,13 +151,15 @@ struct DeviceBatch {
   uint32_t* win_depth = nullptr;       // normal mode, per window: depth | (plain window begins / ends with a stop codon) << 31
 };
 
-enum { CTR_HIST = 0, CTR_SEQ = 1, CTR_NIW = 2, CTR_ERR = 3, CTR_OVF = 4, CTR_VLIST = 5, CTR_SEQD = 6, CTR_NRW = 7, CTR_MERGE = 8, CTR_NREC = 9, CTR_RECSEQ = 10, CTR_HISTD = 11, CTR_NJ = 12, CTR_RPQ = 13, CTR_MQ = 14, CTR_COUNT = 16 };
+enum { CTR_HIST = 0, CTR_SEQ = 1, CTR_NIW = 2, CTR_ERR = 3, CTR_OVF = 4, CTR_VLIST = 5, CTR_SEQD = 6, CTR_NRW = 7, CTR_MERGE = 8, CTR_NREC = 9, CTR_RECSEQ = 10, CTR_HISTD = 11, CTR_NJ = 12, CTR_RPQ = 13, CTR_MQ = 14, CTR_SPILL = 16, CTR_SPQ = 17, CTR_SPQR = 18, CTR_COUNT = 20 };
 
 void launch_read_decode(const DeviceBatch& d, cudaStream_t st);
 void launch_allele_call(const DeviceBatch& d, cudaStream_t st);
 void launch_window_hist(const DeviceBatch& d, cudaStream_t st);
 void launch_replay(const DeviceBatch& d, cudaStream_t st, uint32_t max_ctas = 0);  // replay_kernels.cu; max_ctas: size of the persistent grid (0 = one CTA per unit)
 void launch_window_hist_normal(const DeviceBatch& d, cudaStream_t st);    // normal_kernels.cu (called by launch_window_hist in mode 1)
+enum { SPQ_K2 = 0, SPQ_REPLAY = 1 };  // which queue of the block tier a launch consumes
+void launch_window_hist_block(const DeviceBatch& d, cudaStream_t st, int queue);  // block_kernels.cu
 void launch_assemble_normal(const DeviceBatch& d, cudaStream_t st);
 enum { ASM_ALL = 0, ASM_DEVICE_CLASS = 1, ASM_HOST_CLASS = 2 };  // which end of the key arena a K3 launch walks
 void launch_assemble(const DeviceBatch& d, cudaStream_t st, int part = ASM_ALL);

@@ -131,7 +131,7 @@ __global__ void __launch_bounds__(RC_THREADS, 3) k_rc_count(const DeviceBatch d)
       const uint32_t i = w - sg.win_base;
       uint32_t err = 0;
       n = mph_rc_window_count(c, sg, i, w, d.rw_stopq[x], &bytes, &err);
-      if (n > 0xFFFu) { err |= MPH_E_REC_OVERFLOW; n = 0; }
+      if (n > 0xFFFu) { err |= MPH_E_RECS_PER_LIST; n = 0; }
       // junction merge (:1497-1908): the transcript is still alive after the first window of a later exon; k_rc_merge does it
       const bool junction = i == 0 && !(sg.flags & MPH_SF_FIRST_EXON) && (sg.flags & MPH_SF_JOIN_HEAD) && w < stop && si > 0 && d.segs[si - 1].tx == sg.tx;
       if (junction) d.rw_junc[atomicAdd(&d.counters[CTR_NJ], 1u)] = x;
@@ -228,7 +228,7 @@ __global__ void __launch_bounds__(RM_WARPS * 32, 8) k_rc_merge(const DeviceBatch
       err |= MPH_E_REC_OVERFLOW;
     }
   }
-  if (nm > 0xFFFu) { err |= MPH_E_REC_OVERFLOW; nm = 0; }
+  if (nm > 0xFFFFFu) { err |= MPH_E_RECS_PER_LIST; nm = 0; }  // rw_info keeps 20 bits for them
   if (lane == 0) {
     d.rw_info[x] |= nm << 12;
     d.rw_mbase[x] = mbase;
@@ -327,7 +327,7 @@ __global__ void __launch_bounds__(RC_THREADS) k_nrc_count(const DeviceBatch d) {
         const uint32_t i = w - sg.win_base;
         uint32_t err = 0;
         cnt = mph_nrc_window_count(c, n, sg, i, w, &bytes, &err);
-        if (cnt > 0xFFFu) { err |= MPH_E_REC_OVERFLOW; cnt = 0; }
+        if (cnt > 0xFFFu) { err |= MPH_E_RECS_PER_LIST; cnt = 0; }
         const bool junction = i == 0 && !(sg.flags & MPH_SF_FIRST_EXON) && w < stop && si > 0 && d.segs[si - 1].tx == sg.tx;
         if (junction) d.rw_junc[atomicAdd(&d.counters[CTR_NJ], 1u)] = x;
         raise(d, err);
@@ -365,7 +365,7 @@ __global__ void __launch_bounds__(RM_WARPS * 32) k_nrc_merge(const DeviceBatch d
       err |= MPH_E_REC_OVERFLOW;
     }
   }
-  if (nm > 0xFFFu) { err |= MPH_E_REC_OVERFLOW; nm = 0; }
+  if (nm > 0xFFFFFu) { err |= MPH_E_RECS_PER_LIST; nm = 0; }  // rw_info keeps 20 bits for them
   if (lane == 0) {
     d.rw_info[x] |= nm << 12;
     d.rw_mbase[x] = mbase;

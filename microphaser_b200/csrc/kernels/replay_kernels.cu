@@ -16,6 +16,8 @@ namespace {
 // them. The observation list lives in shared memory (it spills to a global scratch slice if a
 // window is deeper than RP_OBS), the segment's variant positions are cached in shared memory, and
 // the read cursors move incrementally, so an iteration costs one global round trip.
+static_assert((int)MPH_RP_CTR_HIST == (int)CTR_HIST && (int)MPH_RP_CTR_ERR == (int)CTR_ERR && (int)MPH_RP_CTR_VLIST == (int)CTR_VLIST,
+              "mph_replay_tx counts in the kernels' counter words");
 constexpr int RP_WARPS = 1;
 constexpr int RP_OBS = 512;
 constexpr int RP_READS = 640;  // reads of one exon's candidate range cached in shared memory (single-exon units)
@@ -63,6 +65,7 @@ __device__ __forceinline__ void replay_unit(const DeviceBatch& d, const uint32_t
   c.mode = 0; c.tx_id_bytes = nullptr; c.tx_id_off = nullptr; c.win_depth = nullptr; c.win_id = nullptr; c.o_last = nullptr; c.seg_err = d.seg_err;
   c.o_read = nullptr; c.o_hap = nullptr; c.o_frame = nullptr; c.o_flags = nullptr; c.o_inmat = d.o_inmat;
   c.win_out = d.win_out; c.hist = d.hist; c.hist_win = d.hist_win; c.hist_cap = d.hist_cap;
+  c.key_cap = d.force_wide == 2 ? 0u : (uint32_t)MPH_RP_KEYS;
   c.hap0 = d.hap0; c.win_flag = d.win_flag; c.win_voff = d.win_voff; c.vlist = d.vlist; c.vlist_cap = d.vlist_cap;
   c.counters = d.counters; c.sum_depth = d.sum_depth;
   // observation list: shared memory first, generic pointers so that it can move to the global scratch slice
@@ -100,6 +103,7 @@ __device__ __forceinline__ void replay_unit(const DeviceBatch& d, const uint32_t
     for (uint32_t x = lane; x < t.obs_cap; x += 32) in_mat[t.read_lo + x] = 0;
   uint32_t err = 0, ncols = t.dq_n <= MPH_RP_MAXCOLS ? t.dq_n : 0u, n_obs = 0;
   if (t.dq_n > MPH_RP_MAXCOLS) err |= MPH_E_VARS_PER_WINDOW;
+  const uint32_t key_cap = d.force_wide == 2 ? 0u : (uint32_t)MPH_RP_KEYS;
   for (uint32_t j = lane; j < ncols; j += 32) sh.dq[j] = d.dq_init[t.dq_off + j];
   uint64_t last_window_vars = t.last_vars;
   uint32_t cur_lo = r_lo, cur_hi = r_lo;
@@ -378,7 +382,8 @@ __device__ __forceinline__ void replay_unit(const DeviceBatch& d, const uint32_t
         emit_k += sg.k_stride;
         ++emit_i;
         const uint32_t widx = sg.win_base + i;
-        uint32_t n_keys = 0, c0 = 0;
+        uint32_t n_keys = 0, c0 = 0, n_spill = 0;
+        bool spill = false;  // lane 0: a key did not fit the table (the window goes to k_window_hist_block)
         for (uint32_t base = 0; base < n_obs; base += 32) {
           const uint32_t o = base + lane;
           const bool valid = o < n_obs && !(o_flags[o] & 1);
@@ -387,30 +392,62 @@ __device__ __forceinline__ void replay_unit(const DeviceBatch& d, const uint32_t
           const bool zero_key = valid && hap == 0 && fr == 0;
           c0 += __popc(__ballot_sync(FULL, zero_key));
           unsigned pending = __ballot_sync(FULL, valid && !zero_key);
+          n_spill += __popc(pending);
+          if (__shfl_sync(FULL, (int)spill, 0)) continue;
           while (pending) {
             const int leader = __ffs(pending) - 1;
             const uint64_t lh = __shfl_sync(FULL, hap, leader);
             const uint32_t lf = __shfl_sync(FULL, fr, leader);
             const unsigned same = __ballot_sync(FULL, valid && !zero_key && hap == lh && fr == lf);
-            if (lane == 0) {
+            if (lane == 0 && !spill) {
               uint32_t x = 0;
               for (; x < n_keys; ++x)
                 if (sh.table[x].hap == lh && sh.table[x].frame == lf) break;
               if (x == n_keys) {
-                if (n_keys < MPH_RP_KEYS) {
+                if (n_keys < key_cap) {
                   sh.table[x].hap = lh; sh.table[x].frame = lf; sh.table[x].count = 0;
                   ++n_keys;
                 } else {
-                  err |= MPH_E_KEYS_PER_WINDOW;
-                  x = MPH_RP_KEYS - 1;
+                  spill = true;
                 }
               }
-              sh.table[x].count += __popc(same);
+              if (!spill) sh.table[x].count += __popc(same);
             }
             pending &= ~same;
           }
         }
         n_keys = __shfl_sync(FULL, n_keys, 0);
+        if (__shfl_sync(FULL, (int)spill, 0)) {
+          // the counted observations outside the (0, 0) key go to the spill arena; the window to the replay's queue
+          uint32_t off = 0;
+          if (lane == 0) off = atomicAdd(&d.counters[CTR_SPILL], n_spill);
+          off = __shfl_sync(FULL, off, 0);
+          if ((uint64_t)off + n_spill <= d.spill_cap) {
+            uint32_t y = off;
+            for (uint32_t base = 0; base < n_obs; base += 32) {
+              const uint32_t o = base + lane;
+              const bool valid = o < n_obs && !(o_flags[o] & 1);
+              const uint64_t hap = valid ? o_hap[o] : 0;
+              const uint32_t fr = valid ? o_frame[o] : 0;
+              const bool emit = valid && !(hap == 0 && fr == 0);
+              const unsigned bal = __ballot_sync(FULL, emit);
+              if (emit) {
+                MphHist e;
+                e.hap = hap; e.count = 1; e.frame = fr;
+                d.spill[y + __popc(bal & ((1u << lane) - 1u))] = e;
+              }
+              y += __popc(bal);
+            }
+            if (lane == 0) {
+              MphSpillWin q;
+              q.code = ((d.seg_chunk0[si] + (i >> 5)) << 5) | (i & 31u); q.off = off; q.n = n_spill; q.devrec = 0;  // replayed transcripts are host class
+              d.spq_rp[atomicAdd(&d.counters[CTR_SPQR], 1u)] = q;
+            }
+          } else {
+            err |= MPH_E_SPILL_OVERFLOW;
+          }
+          n_keys = 0;  // k_window_hist_block writes the keys and sets n_extra / extra_off
+        }
         if (vl_cur + ncols + 1 > vl_end) {  // a fresh slice of the column-list arena (one atomic per ~256 entries)
           uint32_t got = 0;
           const uint32_t want = max(256u, ncols + 1);
@@ -509,6 +546,7 @@ __global__ void __launch_bounds__(64) k_replay_normal(const DeviceBatch d) {
   c.mode = 1; c.tx_id_bytes = d.tx_id_bytes; c.tx_id_off = d.tx_id_off; c.win_depth = d.win_depth; c.win_id = d.win_id; c.o_last = d.o_key;
   c.o_read = d.o_read; c.o_hap = d.o_hap; c.o_frame = d.o_frame; c.o_flags = d.o_flags; c.o_inmat = d.o_inmat;
   c.win_out = d.win_out; c.hist = d.hist; c.hist_win = d.hist_win; c.hist_cap = d.hist_cap;
+  c.key_cap = d.force_wide == 2 ? 0u : (uint32_t)MPH_RP_KEYS;
   c.hap0 = d.hap0; c.win_flag = d.win_flag; c.win_voff = d.win_voff; c.vlist = d.vlist; c.vlist_cap = d.vlist_cap;
   c.seg_err = d.seg_err; c.counters = d.counters; c.sum_depth = d.sum_depth;
   mph_replay_tx(c, d.replay[ti]);
@@ -517,8 +555,11 @@ __global__ void __launch_bounds__(64) k_replay_normal(const DeviceBatch d) {
 }  // namespace
 
 void launch_replay(const DeviceBatch& d, cudaStream_t st, uint32_t max_ctas) {
-  if (d.rp1 > d.rp0 && d.mode == 1) MPH_LAUNCH(k_replay_normal, ((d.rp1 - d.rp0 + 1) / 2, 64, 0, st), d);
-  else if (d.rp1 > d.rp0) MPH_LAUNCH(k_replay, (std::min<uint32_t>((d.rp1 - d.rp0 + RP_WARPS - 1) / RP_WARPS, max_ctas ? max_ctas : 0xFFFFFFFFu), RP_WARPS * 32, 0, st), d);
+  if (d.rp1 <= d.rp0) return;
+  if (d.mode == 1) MPH_LAUNCH(k_replay_normal, ((d.rp1 - d.rp0 + 1) / 2, 64, 0, st), d);
+  else MPH_LAUNCH(k_replay, (std::min<uint32_t>((d.rp1 - d.rp0 + RP_WARPS - 1) / RP_WARPS, max_ctas ? max_ctas : 0xFFFFFFFFu), RP_WARPS * 32, 0, st), d);
+  // somatic: replayed windows with more keys than the warp's table holds (the normal-mode replay sorts them in the key arena)
+  if (d.mode == 0) launch_window_hist_block(d, st, SPQ_REPLAY);
 }
 
 }  // namespace mphk

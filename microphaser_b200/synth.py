@@ -54,6 +54,8 @@ class Params:
         self.transcripts_per_gene = 1
         self.antisense_frac = 0.0      # chance that an additional transcript of a gene is annotated on the opposite strand
         self.variants_in_introns = True
+        self.independent_somatic = False  # each somatic variant gets its own draw per read (else one draw per read for all of them)
+        self.hotspot_per_gene = 0         # extra somatic SNVs within one 27-nt stretch of one exon per gene (variant-dense windows)
         for k, v in kw.items():
             if not hasattr(self, k):
                 raise TypeError(k)
@@ -241,6 +243,12 @@ def generate(outdir, p):
                 for somatic in [False] * n_g + [True] * n_s:
                     vp = rng.randint(s, e - 1)
                     _add_variant(rng, p, seq, variants, vp, somatic)
+            if p.hotspot_per_gene:
+                wide = [(s, e) for (s, e) in g["exons"] if e - s >= 27] or list(g["exons"])
+                s, e = rng.choice(wide)
+                b = rng.randint(s, max(s, e - 27))
+                for vp in rng.sample(range(b, min(b + 27, e)), min(p.hotspot_per_gene, min(b + 27, e) - b)):
+                    _add_variant(rng, p, seq, variants, vp, True, snv_only=True)
             if p.start_loss_frac and rng.random() < p.start_loss_frac:
                 ex = g["exons"][-1] if g["reverse"] else g["exons"][0]
                 vp = (ex[1] - 1 - rng.randint(0, 2)) if g["reverse"] else ex[0] + rng.randint(0, 2)
@@ -303,7 +311,7 @@ def generate(outdir, p):
                     applied = False
                     if vi < len(vpos) and vpos[vi] == rp:
                         ref, alts, somatic, vhap, vaf = variants[rp]
-                        carry = (take_somatic < vaf) if somatic else (vhap == 2 or vhap == hap)
+                        carry = ((rng.random() if p.independent_somatic else take_somatic) < vaf) if somatic else (vhap == 2 or vhap == hap)
                         if carry:
                             alt = alts[(hap + st) % len(alts)]
                             if len(ref) == 1 and len(alt) == 1:
